@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- queries/sec of the knnQueryBatch hot path on BASELINE.json's metric config.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic queries (config 2: 10 000
 queries x 128-D against 1 000 000 x 128-D, l2sqr, k = 10).  Ours: `value` is measured with the
@@ -13,6 +13,9 @@ device (strong scaling of the fixed 1 M-row workload).
 `--impl reference` times the reference's own CPU implementation (oracle/_ref: the unmodified
 NMSLIB sources, OpenMP over queries on all host cores) on a bounded query sample of the same
 workload.  Prints ONE JSON line on rank 0.
+`--dump-outputs DIR` writes the answers of the last timed step of every record (the ids and distances a
+caller of knnQueryBatch receives) to DIR, so that two builds can be compared output for output on the same
+seeded inputs.
 """
 from __future__ import annotations
 
@@ -21,6 +24,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -31,6 +35,41 @@ ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 
 METRIC = "queries/sec (k=10, exact & HNSW recall@10>=0.95) at 1/2/4/8 B200 vs CPU"
+DUMP_LIMIT = 64 << 20       # bytes written by --dump-outputs, all records together
+OUTPUTS = {}                # workload -> (ids, distances) of its last timed step, kept on rank 0 for --dump-outputs
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """DIR/<workload>_ids.npy (float64, every int32 id exactly) and DIR/<workload>_distances.npy (float32), one row per
+    query, and DIR/<workload>_rows.npy, the query rows they hold: all of them, or above DUMP_LIMIT in all the same
+    fraction of every record's rows, chosen with a fixed seed."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    headers = 3 * 128 * len(outputs)                                  # .npy headers
+    need = sum(ids.shape[0] * (12 * ids.shape[1] + 8) for ids, _ in outputs.values())
+    frac = min(1.0, (DUMP_LIMIT - headers) / max(1, need))
+    for name, (ids, dists) in outputs.items():
+        nq = ids.shape[0]
+        rows = np.arange(nq)
+        if frac < 1.0:
+            rows = np.sort(np.random.default_rng(0).choice(nq, int(nq * frac), replace=False))
+            ids, dists = ids[rows], dists[rows]
+        np.save(out / f"{name}_rows.npy", rows.astype(np.float64))
+        np.save(out / f"{name}_ids.npy", ids.astype(np.float64))
+        np.save(out / f"{name}_distances.npy", dists.astype(np.float32))
+
+
+def keep_outputs(name: str, ids, dists, rank: int, world: int, sliced: bool) -> None:
+    """Copy a record's device answers to the host after its timed steps, for --dump-outputs.  sliced: every rank holds
+    the answers of its own slice of the batch (hnsw replicas) and rank 0 joins them; otherwise rank 0 holds them all."""
+    if sliced and world > 1:
+        import torch.distributed as dist
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object((ids.cpu().numpy(), dists.cpu().numpy()), parts, dst=0)
+        if rank == 0:
+            OUTPUTS[name] = (np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts]))
+    elif rank == 0:
+        OUTPUTS[name] = (ids.cpu().numpy(), dists.cpu().numpy())
 
 
 def load_peaks():
@@ -251,6 +290,8 @@ def run_hnsw(args, w, rank, world, local_rank, dev, dist_on, n_steps, with_cpu):
     barrier()
     ms = e0.elapsed_time(e1)
     st1 = idx.stats()
+    if args.dump_outputs:
+        keep_outputs(w["name"], d_ids, d_dists, rank, world, sliced=True)
     q_np = q_host.numpy()
     for _ in range(2):
         idx.knnQueryBatch(q_np, k)
@@ -289,10 +330,12 @@ def run_hnsw(args, w, rank, world, local_rank, dev, dist_on, n_steps, with_cpu):
             # host cores) on the SAME device-built graph, same efSearch, a bounded query sample
             from oracle import oracle as O
             if O.ref_available():
-                path = "/tmp/nb200_bench_c3.hnsw"
-                idx.save(path, False)
                 threads = os.cpu_count() or 1
-                ref = O.RefIndex(w["space"], "hnsw").load(path)
+                ref = O.RefIndex(w["space"], "hnsw")
+                with tempfile.TemporaryDirectory() as tmp:
+                    path = os.path.join(tmp, "c3.hnsw")
+                    idx.save(path, False)
+                    ref.load(path)
                 ref.set_query_params(f"efSearch={ef}")
                 ref.knn(sample[:64], k, threads=threads)
                 t0 = time.perf_counter()
@@ -311,10 +354,6 @@ def run_hnsw(args, w, rank, world, local_rank, dev, dist_on, n_steps, with_cpu):
                        "sample": f"{len(sample)} of {nq} queries, the reference's Hnsw::Search on the same (device-built) "
                                  f"graph at efSearch={ef}; its recall@{k} on that sample: {rec_ref:.4f} (ours: {rec:.4f})"}
                 ref.close()
-                try:
-                    os.remove(path)
-                except OSError:
-                    pass
         line = {
             "metric": METRIC, "value": nq / (ms_per_step * 1e-3), "unit": "queries/s", "n_gpus": world,
             "steps": n_steps, "warmup": args.warmup, "ms_per_step": ms_per_step, "higher_is_better": True,
@@ -357,7 +396,11 @@ def main():
     ap.add_argument("--parity-sample", type=int, default=256, help="queries of the final answer checked against the oracle")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="N > 1: 'peer' = the library's own NVLink peer-memory exchange, 'nccl' = all-gather + merge")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ids and distances of every record's last timed step to DIR as .npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the answers of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -417,7 +460,7 @@ def main():
                 line["workloads"][name] = {"skipped": f"time budget of {args.budget_s:.0f} s spent"}
                 continue
             try:
-                rec = run(name, steps=max(3, min(args.steps, 10)), warmup=3)
+                rec = run(name, warmup=3)
                 for drop in ("metric", "unit", "higher_is_better", "vs_baseline", "data", "n_gpus", "clocks"):
                     rec.pop(drop, None)
                 line["workloads"][name] = rec
@@ -429,7 +472,7 @@ def main():
             and time.perf_counter() - t_start < args.budget_s):
         rec = None
         try:
-            rec = run("c4", steps=max(3, min(args.steps, 10)), warmup=3, cpu=False)
+            rec = run("c4", warmup=3, cpu=False)
         except Exception as e:
             rec = {"error": f"{type(e).__name__}: {e}"}
         if rank == 0 and line is not None and rec is not None:
@@ -443,7 +486,7 @@ def main():
         rec = None
         try:
             args.parity_sample = min(args.parity_sample, 64)
-            rec = run("c5", steps=3, warmup=3, cpu=False)
+            rec = run("c5", warmup=3, cpu=False)
         except Exception as e:
             rec = {"error": f"{type(e).__name__}: {e}"}
         if rank == 0 and line is not None and rec is not None:
@@ -452,6 +495,8 @@ def main():
             line.setdefault("workloads", {})["c5"] = rec
     if rank == 0 and line is not None:
         line["wall_s"] = time.perf_counter() - t_start
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, OUTPUTS)
         print(json.dumps(line))
     if dist_on:
         dist.destroy_process_group()
@@ -554,6 +599,8 @@ def run_seq(args, w, rank, world, local_rank, dev, dist_on, steps, warmup, with_
     e1.record(stream)
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        keep_outputs(w["name"], o_ids if dist_on else d_ids, o_dists if dist_on else d_dists, rank, world, sliced=False)
     if dist_on:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -2,7 +2,7 @@
 
 ctypes loaders for (a) liboracle_knn.so, the plain-C restatement of the reference's
 query path (knn_oracle.c), and (b) oracle/_ref/*.so, the UNMODIFIED reference compiled
-from /root/reference by oracle/Makefile.  Imported only by tests/, by
+by oracle/Makefile from a checkout of it at oracle/reference/.  Imported only by tests/, by
 __graft_entry__.smoke() and by bench.py's cpu_baseline / --impl reference legs; the
 product package never imports this module.
 """
@@ -28,10 +28,9 @@ def _ptr(a, typ):
     return a.ctypes.data_as(typ) if a is not None else None
 
 
-def build(ref: bool = True) -> None:
-    """Compile the C restatement and, when /root/reference is present, oracle/_ref."""
-    targets = ["oracle"] + (["ref"] if ref else [])
-    subprocess.run(["make", "-s", "-C", str(HERE), f"-j{os.cpu_count() or 4}"] + targets, check=True)
+def build() -> None:
+    """Compile the C restatement and, where a checkout of the reference sits at oracle/reference/, oracle/_ref."""
+    subprocess.run(["make", "-s", "-C", str(HERE), f"-j{os.cpu_count() or 4}", "oracle", "ref"], check=True)
 
 
 # --------------------------------------------------------------------------- C restatement
@@ -43,7 +42,7 @@ def port():
     if _port is None:
         so = HERE / "liboracle_knn.so"
         if not so.exists():
-            build(ref=False)
+            build()
         L = C.CDLL(str(so))
         for name in ("orc_l2sqr", "orc_l2", "orc_norm_scalar_product", "orc_cosine", "orc_negdot",
                      "orc_hnsw_l2sqr", "orc_hnsw_dot", "orc_l1", "orc_linf", "orc_angular"):

@@ -13,11 +13,11 @@ if str(ROOT) not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    # build the product (.so in-tree) and the C restatement; oracle/_ref only where /root/reference exists
+    # build the product (.so in-tree), the C restatement and, where oracle/reference/ holds the reference, oracle/_ref
     from nmslib_zig_b200 import build as nb_build
     nb_build.build()
     from oracle import oracle as O
-    O.build(ref=Path("/root/reference/build.zig").exists())
+    O.build()
 
 
 def pytest_collection_modifyitems(config, items):

@@ -1,12 +1,12 @@
 """Generate tests/golden/*.npz and *.hnsw from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference compiled into oracle/_ref by
+Needs the reference compiled into oracle/_ref (a checkout of it at oracle/reference/, then
 `make -C oracle ref`):
 
     python tests/golden/make_golden.py
 
-Every fixture holds the inputs AND the reference's outputs, so the GPU box (where
-/root/reference does not exist) can check both the oracle port and the CUDA path against
+Every fixture holds the inputs AND the reference's outputs, so a machine without the
+reference can check both the oracle port and the CUDA path against
 numbers produced by the reference itself.  Two routes are used on purpose:
   * "abi": the as-shipped C ABI of the reference (nmslib_index_create -> create_index on empty
     data -> add_data_point_batch -> initialize_pool -> knn_query_fill), i.e. exactly the call

@@ -3,6 +3,8 @@ heuristic-2 selection + batched back links.  The graph is not the reference's gr
 own from one run to the next), so the gate is recall parity: recall@10 at a given efSearch at or above what a
 graph built by the host builder / by the reference itself reaches, plus the structural invariants of the
 optimized-index layout (checked by searching the SAVED file with the oracle's port of the reference search)."""
+from pathlib import Path
+
 import numpy as np
 import pytest
 
@@ -12,12 +14,12 @@ from nmslib_zig_b200 import synth
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
-needs_ref = pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref not built")
+GOLDEN = Path(__file__).resolve().parent / "golden"
 
 
-def _build(space, data, where, extra=None, dtype="DenseVector", dist="Float"):
+def _build(space, data, where, extra=None, dtype="DenseVector", dist="Float", ids=None):
     idx = nb.Index(space, None, "hnsw", dtype, dist)
-    (idx.addUInt8Batch if dtype == "DenseUInt8Vector" else idx.addDenseBatch)(data)
+    (idx.addUInt8Batch if dtype == "DenseUInt8Vector" else idx.addDenseBatch)(data, ids)
     p = {"M": 16, "efConstruction": 200, "b200_build": where}
     p.update(extra or {})
     idx.buildIndex(nb.Params(p))
@@ -95,17 +97,25 @@ def test_device_built_graph_structure(tmp_path):
     g.deinit()
 
 
-@needs_ref
 def test_device_built_graph_recall_vs_reference_built(tmp_path):
-    n, dim = 30_000, 64
-    data, q = synth.gist_like(n, dim, 5, clusters=32), synth.gist_like(400, dim, 6, clusters=32)
-    exact, _, _ = O.seq_knn("l2", data, q, 10)
-    ref = O.RefIndex("l2", "hnsw").add(data).build("M=16,efConstruction=200,indexThreadQty=8")
-    path = tmp_path / "ref.hnsw"
-    ref.save(path)
+    """The reference's graph is built here and now where oracle/_ref exists; elsewhere it is the one the reference built
+    and saved as tests/golden/hnsw_l2_d32.hnsw (rows and ids regenerated as make_golden.py made them)."""
+    if O.ref_available():
+        n, dim = 30_000, 64
+        data, q = synth.gist_like(n, dim, 5, clusters=32), synth.gist_like(400, dim, 6, clusters=32)
+        ids, params = None, None
+        ref = O.RefIndex("l2", "hnsw").add(data).build("M=16,efConstruction=200,indexThreadQty=8")
+        path = tmp_path / "ref.hnsw"
+        ref.save(path)
+    else:
+        data, q = synth.gist_like(2000, 32, 41, clusters=16), synth.gist_like(1000, 32, 43, clusters=16)
+        ids, params = np.arange(2000, dtype=np.int32) + 1000, {"M": 8, "efConstruction": 100}
+        path = GOLDEN / "hnsw_l2_d32.hnsw"
+    exact, _, _ = O.seq_knn("l2", data, q, 10, ids)
     on_ref = nb.Index("l2", None, "hnsw")
     on_ref.importHnsw(path)
-    dev = _build("l2", data, "device")
+    assert np.array_equal(on_ref.getDataPoint(len(data) - 1), data[-1])
+    dev = _build("l2", data, "device", params, ids=ids)
     r_ref, r_dev = _sweep(on_ref, q, exact), _sweep(dev, q, exact)
     for ef, a, b in zip((20, 50, 100, 400), r_dev, r_ref):
         assert a >= b - 0.01, f"ef={ef}: device-built recall {a} < reference-built {b}"
