@@ -282,8 +282,31 @@ typedef struct {
   uint64_t split_queries;    /* queries re-run by the 3xTF32 (split operand) scan after a failed certificate */
   uint64_t u8_imma;          /* 1: uint8 rows are scanned on the integer tensor pipe (tcgen05.mma.kind::i8), 0: widened to TF32 */
   uint64_t uploaded_rows;    /* rows copied host -> device so far (an append uploads only the new rows) */
+  /* nmslib_b200_range_query_batch (b200_devices indexes: counted once per shard) */
+  uint64_t range_tc_queries;       /* range queries whose answer came from the tensor-core pass */
+  uint64_t range_fallback_queries; /* range queries re-run by the per-query exact scan (tensor-core pass uncertified) */
 } nmslib_b200_stats_t;
 nmslib_error_t nmslib_b200_get_stats(nmslib_index_handle_t index, nmslib_b200_stats_t* out);
+
+/* Batched range queries (seq_search / brute_force).  `queries` is laid out like the input of
+ * nmslib_knn_query_batch (query_count x elem_count floats, or bytes for uint8 indexes); radii[i] is query i's
+ * radius and results[i] a caller-owned slot of results[i].capacity entries; results[i].size is set on return.
+ * For every query the answer is exactly what nmslib_range_query_fill returns for it with radii[i] and
+ * results[i].capacity: the objects within the radius in position order, truncated to the capacity, with the same
+ * distance bits and the same radius conversions ((float)radius; floor for l2sqr_sift, RangeQuery<int>).
+ * Errors: a negative radius, a NULL pointer or a capacity of 0 anywhere in the batch -> INVALID_ARGUMENT before
+ * any work; a query length that does not match the index -> QUERY_EXECUTION_FAILED; hnsw -> SPACE_INCOMPATIBLE
+ * (the reference has no range search over hnsw); an index that is not built -> INDEX_BUILD_FAILED, as for
+ * nmslib_range_query_fill.  An empty index returns size 0 everywhere.
+ * l2, l2sqr, cosinesimil, negdotprod and angulardist run as one tensor-core pass over the rows for the whole batch
+ * (a threshold per query, verified with the per-query scan's own distance code); l1, linf, uint8 indexes
+ * (l2sqr_sift: the integer-pipe kernel has no range mode yet), force_exact and, under option tc_pair=0, rows of more
+ * than 128 floats use the per-query exact scan, as does
+ * any query the tensor-core pass cannot certify (nmslib_b200_stats_t counts both).  A b200_devices index answers
+ * over every shard and concatenates the shards' lists in position order. */
+nmslib_error_t nmslib_b200_range_query_batch(nmslib_index_handle_t index, const void* queries,
+                                             size_t query_count, size_t elem_count,
+                                             const double* radii, nmslib_result_t* results);
 
 /* Diagnostic (needs no device): the work decomposition the tensor-core scan would use for a batch of
  * `query_count` queries against `n` rows of at most 128 floats on a GPU with `sm_count` SMs.

@@ -528,6 +528,38 @@ nmslib_error_t nmslib_range_query_fill(nmslib_index_handle_t index, const void* 
       },
       NMSLIB_ERROR_QUERY_EXECUTION_FAILED, "Range query failed");
 }
+nmslib_error_t nmslib_b200_range_query_batch(nmslib_index_handle_t index, const void* queries, size_t query_count,
+                                             size_t elem_count, const double* radii, nmslib_result_t* results) {
+  // the whole batch is checked before any work (codes of nmslib_range_query_get_size / _fill)
+  if (!index || !queries || query_count == 0 || !radii || !results)
+    return NB_ERR(NMSLIB_ERROR_INVALID_ARGUMENT, "Invalid range batch inputs");
+  for (size_t i = 0; i < query_count; ++i) {
+    if (radii[i] < 0) return NB_ERR(NMSLIB_ERROR_INVALID_ARGUMENT, "Negative radius in range batch");
+    if (!results[i].ids || !results[i].distances || results[i].capacity == 0)
+      return NB_ERR(NMSLIB_ERROR_INVALID_ARGUMENT, "Result buffers invalid");
+  }
+  return guarded(
+      [&]() -> nmslib_error_t {
+        Engine* e = index->engine;
+        std::lock_guard<std::mutex> lock(e->mutex());
+        std::vector<size_t> caps(query_count), sizes(query_count, 0);
+        std::vector<int32_t*> ids(query_count);
+        std::vector<float*> dists(query_count);
+        for (size_t i = 0; i < query_count; ++i) {
+          caps[i] = results[i].capacity;
+          ids[i] = results[i].ids;
+          dists[i] = results[i].distances;
+        }
+        Status s = index->group ? index->group->range_host(e, queries, query_count, elem_count, radii, caps.data(),
+                                                           ids.data(), dists.data(), sizes.data())
+                                : e->range_batch_host(queries, query_count, elem_count, radii, caps.data(), ids.data(),
+                                                      dists.data(), sizes.data());
+        for (size_t i = 0; i < query_count; ++i) results[i].size = s.ok() ? sizes[i] : 0;
+        if (!s.ok()) return NB_STATUS(s);
+        return NB_OK("Range query batch executed");
+      },
+      NMSLIB_ERROR_QUERY_EXECUTION_FAILED, "Range query batch failed");
+}
 nmslib_error_t nmslib_get_data_point_string(nmslib_index_handle_t index, size_t, const char** data, size_t* data_len,
                                             const nmslib_allocator_t* allocator) {
   if (!index || !data || !data_len || !alloc_ok(allocator)) return NB_ERR(NMSLIB_ERROR_INVALID_ARGUMENT, "Invalid arguments");
@@ -830,6 +862,8 @@ nmslib_error_t nmslib_b200_get_stats(nmslib_index_handle_t index, nmslib_b200_st
   out->build_prunes = bi.prunes;
   out->split_queries = s.split_queries;
   out->uploaded_rows = s.uploaded_rows;
+  out->range_tc_queries = s.range_tc_queries;
+  out->range_fallback_queries = s.range_fallback_queries;
   out->u8_imma = (!index->group && index->engine->is_u8() && index->engine->method() == nb200::METHOD_SEQ &&
                   index->engine->u8_imma()) ? 1 : 0;
   return NMSLIB_SUCCESS;

@@ -195,6 +195,7 @@ void Engine::release_device() {
   d_fb_cnt_.release();
   d_digits_.release();
   d_glists_.release();
+  for (DevBuf* b : {&d_rq_, &d_rq_out_, &d_rcand_, &d_rcnt_, &d_rcut_, &d_rthr_, &d_rplan_}) b->release();
   upload_valid_ = false;
   n_up_ = 0;
   n_dev_ = 0;
@@ -1357,6 +1358,16 @@ Status Engine::knn_device(const void* d_queries, size_t nq, size_t elem_count, s
   return s;
 }
 
+int Engine::range_mode() const {
+  return dev_u8_rows()             ? SCAN_SIFT  // byte rows (128 per row)
+         : space_ == SPACE_COSINE  ? SCAN_COSINE
+         : space_ == SPACE_ANGULAR ? SCAN_ANGULAR
+         : space_ == SPACE_NEGDOT  ? SCAN_NEGDOT
+         : space_ == SPACE_L1      ? SCAN_L1
+         : space_ == SPACE_LINF    ? SCAN_LINF
+                                   : SCAN_L2;
+}
+
 // SeqSearch::Search(RangeQuery*) (seqsearch.cc:108-141) through nmslib_range_query_fill (nmslib_c.cpp:1051-1153):
 // every object within the radius, in position order, truncated to the caller's capacity.
 Status Engine::range_host(const void* query, size_t elem_count, double radius, size_t capacity, int32_t* ids,
@@ -1380,13 +1391,7 @@ Status Engine::range_host(const void* query, size_t elem_count, double radius, s
   int32_t* d_ids = reinterpret_cast<int32_t*>(d_range_.as<char>() + tmp_bytes);
   float* d_d = reinterpret_cast<float*>(d_range_.as<char>() + tmp_bytes + out_bytes);
   int* d_cnt = reinterpret_cast<int*>(d_range_.as<char>() + tmp_bytes + 2 * out_bytes);
-  const int mode = dev_u8_rows()             ? SCAN_SIFT  // byte rows (128 per row)
-                   : space_ == SPACE_COSINE  ? SCAN_COSINE
-                   : space_ == SPACE_ANGULAR ? SCAN_ANGULAR
-                   : space_ == SPACE_NEGDOT  ? SCAN_NEGDOT
-                   : space_ == SPACE_L1      ? SCAN_L1
-                   : space_ == SPACE_LINF    ? SCAN_LINF
-                                             : SCAN_L2;
+  const int mode = range_mode();
   // RangeQuery<int> compares with static_cast<int>(radius) (nmslib_c.cpp:1087-1088)
   const float r = is_u8_ ? std::floor((float)radius) : (float)radius;
   s = check_cuda(launch_range_scan(d_db_.as<float>(), d_q_.as<float>(),
@@ -1409,6 +1414,199 @@ Status Engine::range_host(const void* query, size_t elem_count, double radius, s
   *size = (size_t)found;
   stats_.queries += 1;
   stats_.distance_evals += n_dev_;
+  return Status::OK();
+}
+
+// Batched range queries (K5b, DESIGN.md): the answer of range_host for every query, one device submission per chunk.
+// Float spaces with a dot-product form run on the tensor cores: radius -> pass-1 threshold T_q, the TS / pair scan
+// in range mode (survivors of rank < T_q in position order, a position cut where a list fills), verification of the
+// candidates with the per-query scan's own distance code.  l1 / linf / uint8 / force_exact, and every query the
+// tensor-core pass cannot certify, take the per-query exact scan (launch_range_scan) inside the same submission.
+// Outputs are staged in CSR form (min(capacity, n) slots per query); a batch whose staging would exceed
+// kRangeStageBytes runs in query chunks.
+namespace {
+constexpr size_t kRangeStageBytes = 64u << 20;  // ids + distances staged on the device per chunk
+constexpr size_t kRangeChunkQueries = 65536;    // bounds the candidate lists of one chunk as well
+}  // namespace
+
+Status Engine::range_batch_host(const void* queries, size_t nq, size_t elem_count, const double* radii,
+                                const size_t* caps, int32_t* const* ids, float* const* dists, size_t* sizes) {
+  for (size_t i = 0; i < nq; ++i) sizes[i] = 0;
+  if (!built_) return Status::Err(kErrBuild, "Index not built");
+  if (method_ != METHOD_SEQ)
+    return Status::Err(kErrIncompat, "Range query not supported by method: Range search is not supported!");
+  Status s = prepare();
+  if (!s.ok()) return s;
+  if (n_dev_ == 0 || nq == 0) return Status::OK();
+  if (elem_count != (size_t)dim_)
+    return Status::Err(kErrQuery, "query length " + std::to_string(elem_count) + " != index dimension " +
+                                      std::to_string(dim_));
+  // the radius conversions of range_host (RangeQuery<int> compares with static_cast<int>(radius))
+  std::vector<float> r(nq);
+  std::vector<int> cap(nq);
+  for (size_t i = 0; i < nq; ++i) {
+    r[i] = is_u8_ ? std::floor((float)radii[i]) : (float)radii[i];
+    cap[i] = (int)std::min<size_t>(caps[i], n_dev_);
+  }
+  const size_t esz = is_u8_ ? 1 : 4;
+  size_t c0 = 0;
+  while (c0 < nq) {
+    size_t c1 = c0, staged = 0;
+    while (c1 < nq && c1 - c0 < kRangeChunkQueries &&
+           (c1 == c0 || (staged + (size_t)cap[c1]) * 8 <= kRangeStageBytes))
+      staged += (size_t)cap[c1++];
+    s = range_chunk(static_cast<const char*>(queries) + c0 * elem_count * esz, c1 - c0, elem_count, r.data() + c0,
+                    cap.data() + c0, ids + c0, dists + c0, sizes + c0);
+    if (!s.ok()) return s;
+    c0 = c1;
+  }
+  stats_.queries += nq;
+  stats_.distance_evals += (uint64_t)nq * n_dev_;
+  return Status::OK();
+}
+
+Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, const float* radii, const int* caps,
+                           int32_t* const* ids, float* const* dists, size_t* sizes) {
+  const int mode = range_mode();
+  const int take_sqrt = space_ == SPACE_L2 ? 1 : 0;
+  // the tensor-core pass needs the TS kernel (rows <= 128 floats) or the pair kernel; with option tc_pair=0 longer
+  // rows take the per-query exact scan like l1 / linf (not counted as fallbacks: no tensor-core pass was made)
+  const bool ts = tc_ts_supported(row_words_);
+  const bool pair = !ts && tc_pair_enabled() && sm_count_ >= 2;
+  const bool tc = !force_exact_ && !is_u8_ && (ts || pair) &&
+                  (space_ == SPACE_L2 || space_ == SPACE_L2SQR || space_ == SPACE_COSINE || space_ == SPACE_NEGDOT ||
+                   space_ == SPACE_ANGULAR);
+  Status s = stage_queries_device(queries, false, nq, elem_count, stream_);
+  if (!s.ok()) return s;
+  // per-query parameters: radii [nq] f32 | caps [nq] i32 | CSR offsets [nq] i64; outputs: counts [nq] | fallback
+  // count [1] + list [nq] | ids [total] | distances [total]
+  std::vector<int64_t> off(nq);
+  int64_t total = 0;
+  for (size_t i = 0; i < nq; ++i) {
+    off[i] = total;
+    total += caps[i];
+  }
+  const size_t a4 = round_up(nq * 4, 256), a8 = round_up(nq * 8, 256);
+  std::vector<char> h_par(2 * a4 + a8);
+  memcpy(h_par.data(), radii, nq * 4);
+  memcpy(h_par.data() + a4, caps, nq * 4);
+  memcpy(h_par.data() + 2 * a4, off.data(), nq * 8);
+  if (!(s = check_cuda(d_rq_.ensure(h_par.size()), "cudaMalloc(range params)")).ok()) return s;
+  s = check_cuda(cudaMemcpyAsync(d_rq_.p, h_par.data(), h_par.size(), cudaMemcpyHostToDevice, stream_), "H2D(range params)");
+  if (!s.ok()) return s;
+  const float* d_radii = d_rq_.as<float>();
+  const int* d_caps = reinterpret_cast<const int*>(d_rq_.as<char>() + a4);
+  const int64_t* d_off = reinterpret_cast<const int64_t*>(d_rq_.as<char>() + 2 * a4);
+  const size_t ob = round_up((size_t)total * 4, 256);
+  if (!(s = check_cuda(d_rq_out_.ensure(3 * a4 + 256 + 2 * ob), "cudaMalloc(range outputs)")).ok()) return s;
+  int* d_counts = d_rq_out_.as<int>();
+  int* d_fb_cnt = reinterpret_cast<int*>(d_rq_out_.as<char>() + a4);
+  int* d_fb_idx = reinterpret_cast<int*>(d_rq_out_.as<char>() + a4 + 256);
+  int32_t* d_oids = reinterpret_cast<int32_t*>(d_rq_out_.as<char>() + 2 * a4 + 256);
+  float* d_odists = reinterpret_cast<float*>(d_rq_out_.as<char>() + 2 * a4 + 256 + ob);
+  if (!(s = check_cuda(d_range_.ensure(round_up(n_dev_ * 4, 256)), "cudaMalloc(range)")).ok()) return s;
+  const float* aux = (mode == SCAN_COSINE || mode == SCAN_ANGULAR) ? d_aux_.as<float>() : nullptr;
+  // the per-query exact scan of query i (every query of the chunk, or the uncertified ones)
+  auto exact = [&](size_t i) {
+    stats_.kernel_launches += 2;
+    return check_cuda(launch_range_scan(d_db_.as<float>(), reinterpret_cast<const float*>(d_q_.as<char>() + i * row_words_ * 4),
+                                        aux, d_ids_.as<int32_t>(), (int)n_dev_, row_words_, mode, take_sqrt, radii[i],
+                                        caps[i], d_range_.as<float>(), d_oids + off[i], d_odists + off[i], d_counts + i,
+                                        stream_),
+                      "range_scan");
+  };
+  size_t n_fb = 0;
+  if (!tc) {
+    for (size_t i = 0; i < nq && s.ok(); ++i) s = exact(i);
+    if (!s.ok()) return s;
+  } else {
+    const int qb = tc_block_queries();
+    const size_t q_pad = round_up(nq, (size_t)qb);
+    const size_t n_pad = round_up(n_dev_, (size_t)tc_block_points());
+    int n_cta, slots;
+    if (ts) tc_ts_plan((int)nq, (int)n_dev_, 1, sm_count_, &h_rplan_, &n_cta, &slots);
+    else tc_ts_plan((int)nq, (int)n_dev_, 1, sm_count_ / 2, &h_rplan_, &n_cta, &slots, tc_pair_block_points(), 2);
+    const int s_max = pair ? 2 * slots : slots;
+    const size_t lists = q_pad / qb * (size_t)s_max * qb, cap = (size_t)tc_range_cap();
+    if (!(s = check_cuda(d_rplan_.ensure(h_rplan_.size() * 4), "cudaMalloc(range plan)")).ok()) return s;
+    s = check_cuda(cudaMemcpyAsync(d_rplan_.p, h_rplan_.data(), h_rplan_.size() * 4, cudaMemcpyHostToDevice, stream_),
+                   "H2D(range plan)");
+    if (!s.ok()) return s;
+    if (!(s = check_cuda(d_rcand_.ensure(lists * cap * 8), "cudaMalloc(range cand)")).ok()) return s;
+    if (!(s = check_cuda(d_rcnt_.ensure(lists * 4), "cudaMalloc(range cand_cnt)")).ok()) return s;
+    if (!(s = check_cuda(d_rcut_.ensure(lists * 4), "cudaMalloc(range cut)")).ok()) return s;
+    if (!(s = check_cuda(d_rthr_.ensure(q_pad * 4), "cudaMalloc(range thr)")).ok()) return s;
+    if (!(s = check_cuda(cudaMemsetAsync(d_rcnt_.p, 0xFF, lists * 4, stream_), "memset(range cand_cnt)")).ok()) return s;
+    if (!(s = check_cuda(cudaMemsetAsync(d_fb_cnt, 0, 4, stream_), "memset(range fb count)")).ok()) return s;
+    const int tmode = space_ == SPACE_COSINE ? SCAN_COSINE : space_ == SPACE_ANGULAR ? SCAN_ANGULAR
+                      : space_ == SPACE_NEGDOT ? SCAN_NEGDOT : SCAN_L2;
+    s = check_cuda(launch_tc_range_threshold(d_q_.as<float>(), (int)nq, row_words_, tmode, take_sqrt, d_radii, x_max_,
+                                             db_inexact_ ? 1 : 0, d_rthr_.as<uint32_t>(), stream_),
+                   "tc_range_threshold");
+    if (!s.ok()) return s;
+    // pass 1 on the plain operands (never the split copy): the threshold's error band covers TF32-inexact data
+    const bool cosf = tmode == SCAN_COSINE || tmode == SCAN_ANGULAR;
+    const float scale = tmode == SCAN_L2 ? -2.f : -1.f;
+    const float* dbB = cosf ? d_db_unit_.as<float>() : d_db_.as<float>();
+    const float* nbp = tmode == SCAN_L2 ? d_nblock_.as<float>() : nullptr;
+    if (pair) {
+      if (!(s = check_cuda(d_qa_.ensure(q_pad * (size_t)row_words_ * 4), "cudaMalloc(qa)")).ok()) return s;
+      s = check_cuda(launch_tc_prep_queries(d_q_.as<float>(), d_qa_.as<float>(), q_pad * (size_t)row_words_, scale,
+                                            d_flags_.as<int>() + 1, stream_),
+                     "tc_prep_queries");
+      if (!s.ok()) return s;
+      ++stats_.kernel_launches;
+    }
+    scan_begin(stream_);
+    s = check_cuda(ts ? launch_tc_scan_ts(d_q_.as<float>(), dbB, n_pad, nbp, d_ones_.as<float>(), (int)n_dev_, (int)nq,
+                                          row_words_, 1, 0, scale, pos_base_, n_cta, s_max, d_rplan_.as<int>(),
+                                          d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), nullptr, d_rthr_.as<uint32_t>(),
+                                          d_flags_.as<int>() + 1, stream_, d_rcut_.as<uint32_t>())
+                      : launch_tc_scan_pair(d_qa_.as<float>(), q_pad, dbB, n_pad, nbp, d_ones_.as<float>(), (int)n_dev_,
+                                            (int)nq, row_words_, 1, pos_base_, n_cta, d_rplan_.as<int>(), s_max, 0,
+                                            d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), nullptr, d_rthr_.as<uint32_t>(),
+                                            stream_, d_rcut_.as<uint32_t>()),
+                   ts ? "tc_scan_ts(range)" : "tc_scan_pair(range)");
+    scan_end(stream_);
+    if (!s.ok()) return s;
+    s = check_cuda(launch_range_verify(d_db_.as<float>(), d_q_.as<float>(), d_ids_.as<int32_t>(), row_words_, mode,
+                                       take_sqrt, pos_base_, d_radii, d_caps, d_off, d_rcand_.as<uint64_t>(),
+                                       d_rcnt_.as<int>(), d_rcut_.as<uint32_t>(), s_max, (int)cap, 0, (int)nq, d_oids,
+                                       d_odists, d_counts, d_fb_cnt, d_fb_idx, stream_),
+                   "range_verify");
+    if (!s.ok()) return s;
+    stats_.kernel_launches += 3;
+    int fb_cnt = 0;
+    s = check_cuda(cudaMemcpyAsync(&fb_cnt, d_fb_cnt, 4, cudaMemcpyDeviceToHost, stream_), "D2H(range fb count)");
+    if (s.ok()) s = check_cuda(cudaStreamSynchronize(stream_), "range batch");
+    if (!s.ok()) return s;
+    n_fb = (size_t)fb_cnt;
+    if (n_fb > 0) {
+      std::vector<int> fb(n_fb);
+      s = check_cuda(cudaMemcpyAsync(fb.data(), d_fb_idx, n_fb * 4, cudaMemcpyDeviceToHost, stream_), "D2H(range fb list)");
+      if (s.ok()) s = check_cuda(cudaStreamSynchronize(stream_), "range batch");
+      for (size_t j = 0; j < n_fb && s.ok(); ++j) s = exact((size_t)fb[j]);
+      if (!s.ok()) return s;
+    }
+    stats_.range_tc_queries += nq - n_fb;
+    stats_.range_fallback_queries += n_fb;
+  }
+  std::vector<int> cnt(nq);
+  std::vector<int32_t> h_ids((size_t)total);
+  std::vector<float> h_d((size_t)total);
+  s = check_cuda(cudaMemcpyAsync(cnt.data(), d_counts, nq * 4, cudaMemcpyDeviceToHost, stream_), "D2H(range counts)");
+  if (s.ok() && total > 0)
+    s = check_cuda(cudaMemcpyAsync(h_ids.data(), d_oids, (size_t)total * 4, cudaMemcpyDeviceToHost, stream_), "D2H(range ids)");
+  if (s.ok() && total > 0)
+    s = check_cuda(cudaMemcpyAsync(h_d.data(), d_odists, (size_t)total * 4, cudaMemcpyDeviceToHost, stream_), "D2H(range dists)");
+  if (s.ok()) s = check_cuda(cudaStreamSynchronize(stream_), "range batch");
+  if (!s.ok()) return s;
+  for (size_t i = 0; i < nq; ++i) {
+    const size_t c = (size_t)cnt[i];
+    memcpy(ids[i], h_ids.data() + off[i], c * 4);
+    memcpy(dists[i], h_d.data() + off[i], c * 4);
+    sizes[i] = c;
+  }
   return Status::OK();
 }
 

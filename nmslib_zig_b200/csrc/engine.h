@@ -146,6 +146,7 @@ struct Stats {
   double last_kernel_ms = 0, last_total_ms = 0, last_scan_ms = 0, scan_ms_sum = 0;
   uint64_t scan_count = 0;
   uint64_t fallback_queries = 0, device_bytes = 0, split_queries = 0, uploaded_rows = 0;
+  uint64_t range_tc_queries = 0, range_fallback_queries = 0;  // batched range queries (range_batch_host)
 };
 
 class Engine {
@@ -201,6 +202,10 @@ class Engine {
   // range query of one object (seq_search only, like the reference): ids/dists are caller buffers of `capacity`
   Status range_host(const void* query, size_t elem_count, double radius, size_t capacity, int32_t* ids, float* dists,
                     size_t* size);
+  // a batch of range queries: for every i the answer range_host gives with radii[i] and caps[i], written to the
+  // caller buffers ids[i] / dists[i] (caps[i] entries), sizes[i] = entries written
+  Status range_batch_host(const void* queries, size_t nq, size_t elem_count, const double* radii, const size_t* caps,
+                          int32_t* const* ids, float* const* dists, size_t* sizes);
   // device in / device out
   // src_pitch: bytes between query rows (0 = dense rows of elem_count elements)
   Status knn_device(const void* d_queries, size_t nq, size_t elem_count, size_t k, int32_t* d_ids,
@@ -256,6 +261,10 @@ class Engine {
   Status stage_queries_device(const void* src, bool src_on_device, size_t nq, size_t elem_count,
                               cudaStream_t stream, size_t src_pitch = 0);
   Status build_graph_device();
+  int range_mode() const;  // distance code of range_scan.cu for this index
+  // one chunk of range_batch_host: queries [0, nq) of `queries`, per-query float radii / capacities (<= n)
+  Status range_chunk(const void* queries, size_t nq, size_t elem_count, const float* radii, const int* caps,
+                     int32_t* const* ids, float* const* dists, size_t* sizes);
 
   Space space_;
   Method method_;
@@ -304,6 +313,9 @@ class Engine {
   cudaStream_t copy_stream_ = nullptr;
   cudaEvent_t copy_ev_[kCopyChunks + 1] = {};
   DevBuf d_range_;                      // per-row distances of a range query + its outputs
+  // batched range queries: per-query parameters + CSR outputs, and the range-mode candidate lists of the scan
+  DevBuf d_rq_, d_rq_out_, d_rcand_, d_rcnt_, d_rcut_, d_rthr_, d_rplan_;
+  std::vector<int> h_rplan_;
   DevBuf d_u8tmp_;                      // staging for uint8 rows / queries before they are widened
   DevBuf d_gthr_;                       // per-query threshold shared by the CTAs of one scan
   bool db_inexact_ = false;             // the uploaded rows are not TF32-exact (read back once at upload)

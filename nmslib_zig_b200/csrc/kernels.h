@@ -94,7 +94,8 @@ int tc_pair_block_points();
 cudaError_t launch_tc_scan_pair(const float* qa, size_t q_pad, const float* dbB, size_t n_pad, const float* nblock,
                                 const float* ones, int n, int nq, int row_words, int k, uint32_t pos_base, int n_pairs,
                                 const int* d_pieces, int s_max, int kprime, uint64_t* cand, int* cand_cnt,
-                                float* cand_thr, uint32_t* gthr, cudaStream_t stream);
+                                float* cand_thr, uint32_t* gthr, cudaStream_t stream,
+                                uint32_t* range_cut = nullptr);  // range mode (see launch_tc_scan_ts)
 // rows of at most 128 floats: the prepared queries live in tensor memory (tc_scan_ts_kernel); q = the ORIGINAL
 // queries [q_pad][row_words], scaled on the fly; sets *inexact_flag when a valid query row is not TF32-exact
 bool tc_ts_supported(int row_words);
@@ -109,7 +110,17 @@ void tc_ts_plan(int nq, int n, int k, int sm_count, std::vector<int>* table, int
 cudaError_t launch_tc_scan_ts(const float* q, const float* dbB, size_t n_pad, const float* nblock, const float* ones,
                               int n, int nq, int row_words, int k, int kprime, float scale, uint32_t pos_base,
                               int n_cta, int s_max, const int* d_pieces, uint64_t* cand, int* cand_cnt,
-                              float* cand_thr, uint32_t* gthr, int* inexact_flag, cudaStream_t stream);
+                              float* cand_thr, uint32_t* gthr, int* inexact_flag, cudaStream_t stream,
+                              uint32_t* range_cut = nullptr);
+// Range mode of the two scans above (range_cut != NULL): gthr holds every query's fixed threshold T_q
+// (launch_tc_range_threshold), lists hold tc_range_cap() keys in position order, and range_cut
+// ([q_blocks][s_max][256], written for every list in use instead of cand_thr) receives the position of the first
+// survivor a full list dropped (0xFFFFFFFF = none).  k only shapes the plan.
+int tc_range_cap();
+// mode: SCAN_L2 (take_sqrt: l2, else l2sqr) / SCAN_COSINE / SCAN_ANGULAR / SCAN_NEGDOT; radii: [nq] float radii;
+// q: staged queries [q_pad][row_words]; x_max / db_inexact: as for the re-rank's certificate
+cudaError_t launch_tc_range_threshold(const float* q, int nq, int row_words, int mode, int take_sqrt, const float* radii,
+                                      float x_max, int db_inexact, uint32_t* gthr, cudaStream_t stream);
 cudaError_t launch_tc_prep_queries(const float* q, float* out, size_t words, float scale, int* inexact_flag,
                                    cudaStream_t stream);
 // qa: prepared queries [q_pad][row_words]; dbB: B operand rows [n_pad][row_words];
@@ -147,6 +158,16 @@ cudaError_t launch_tc_split_rows(const float* src, size_t rows, int row_words, f
 cudaError_t launch_range_scan(const float* db, const float* query, const float* db_norm2, const int32_t* ext_ids, int n,
                               int row_words, int mode, int take_sqrt, float radius, int capacity, float* dist_tmp,
                               int32_t* out_ids, float* out_dists, int* out_count, cudaStream_t stream);
+// Batched range queries, verification of the tensor-core candidates (one block per query of [q0, q0 + count)):
+// cand / cand_cnt / cut: the range-mode lists of launch_tc_scan_ts / _pair (s_max lists per 256-query block of
+// list_cap keys); only candidates below the smallest cut are evaluated, with the distance code of launch_range_scan.
+// Outputs in CSR form: query q writes at most caps[q] hits at out_off[q] and *out_count[q]; a query that cannot be
+// certified (a list overflowed and fewer than caps[q] hits lie below the cut) is appended to fb_idx / *fb_count.
+cudaError_t launch_range_verify(const float* db, const float* queries, const int32_t* ext_ids, int row_words, int mode,
+                                int take_sqrt, uint32_t pos_base, const float* radii, const int* caps,
+                                const int64_t* out_off, const uint64_t* cand, const int* cand_cnt, const uint32_t* cut,
+                                int s_max, int list_cap, int q0, int count, int32_t* out_ids, float* out_dists,
+                                int* out_count, int* fb_count, int* fb_idx, cudaStream_t stream);
 
 // ---- hnsw_search.cu ------------------------------------------------------------------
 struct HnswDeviceGraph {

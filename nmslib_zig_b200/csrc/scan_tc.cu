@@ -34,6 +34,9 @@
 // epi_select_tile) go to the row's candidate buffer.  The long-row kernels use the round-1 epilogue (epi_process, 32
 // columns at a time).  Thresholds: the exact 16th best in a register list for k <= 12, otherwise tightened by
 // warp-cooperative compaction of the buffer; shared between the CTAs of one query through a per-query word.
+// Batched range queries (DESIGN.md K5b): the TS and pair kernels have a RANGE variant whose thresholds are fixed per
+// query (tc_range_threshold_kernel turns the radius into the pass-1 rank domain, widened by the certificate's error
+// band); survivors are kept in position order up to a position cut, and range_scan.cu verifies them.
 #include <cuda.h>
 
 #include <algorithm>
@@ -307,11 +310,13 @@ constexpr int TS_RK = 16;  // register mode: ranks of a row's 16 best candidates
 // kept as a sorted register list of RANKS only (insertion = a 16-step min/max chain); the (rank, position) keys
 // themselves are appended to the row's buffer, which then only ever receives the ~k ln(N) true improvements
 // and needs no compaction.  !REG: the threshold tightens when the buffer is compacted (compact_row).
-template <int KPL, bool REG>
+// RANGE (batched range queries): the threshold is the query's fixed T_q; survivors are appended in position order
+// until the buffer is full, then the row records the position of its first dropped survivor in *cut and stops.
+template <int KPL, bool REG, bool RANGE = false>
 __device__ __forceinline__ void epi_process(const uint32_t (&v)[32], uint32_t pos0, int vcols, uint64_t* buf, int& cnt,
                                             float& thr, float (&tk)[TS_RK], int cap, int kprime, int slack,
-                                            uint32_t* gthr, int lane, unsigned (&ctr)[4]) {
-  unsigned need = __ballot_sync(FULL, cnt > cap - 32);
+                                            uint32_t* gthr, int lane, unsigned (&ctr)[4], uint32_t* cut = nullptr) {
+  unsigned need = RANGE ? 0u : __ballot_sync(FULL, cnt > cap - 32);
   while (need) {  // about to overflow: compact at once (!REG: normally the deferred path keeps rows far from here)
     ++ctr[2];
     const int src = __ffs(need) - 1;
@@ -367,6 +372,18 @@ __device__ __forceinline__ void epi_process(const uint32_t (&v)[32], uint32_t po
               }
             }
           }
+        } else if constexpr (RANGE) {
+#pragma unroll
+          for (int j = 8 * q; j < 8 * q + 8; ++j) {
+            if (r[j] < thr) {
+              if (cnt == cap) {  // full: everything kept lies before this position
+                *cut = pos0 + j;
+                thr = __int_as_float(0xFF800000);
+              } else {
+                buf[cnt++] = ((uint64_t)__float_as_uint(r[j]) << 32) | (uint64_t)(pos0 + j);
+              }
+            }
+          }
         } else {
 #pragma unroll
           for (int j = 8 * q; j < 8 * q + 8; ++j) {
@@ -403,10 +420,12 @@ __device__ __forceinline__ float group_min8(const float (&r)[32], int q) {
 // small: ONE copy of the insertion code, walked by bit masks (also measured and rejected: fully unrolled over the 64
 // registers -- 40 KB of code, 2 x slower, stall_no_inst -- and a per-thread scratch array in local memory walked with
 // dynamic indices -- 3 x slower, the stores delay the next tile's tensor-memory drain).
-template <bool REG>
+// RANGE: groups and the values within a group are walked in increasing column order, so the keys are appended in
+// position order and a full buffer records its first dropped position in *cut (see epi_process).
+template <bool REG, bool RANGE = false>
 __device__ __forceinline__ void epi_select_tile(const float (&r0)[32], const float (&r1)[32], const float (&g0)[4],
                                                 const float (&g1)[4], uint32_t pos0, uint64_t* buf, int& cnt, float& thr,
-                                                float (&tk)[TS_RK], uint32_t* gthr) {
+                                                float (&tk)[TS_RK], uint32_t* gthr, int cap = 0, uint32_t* cut = nullptr) {
   unsigned gm = 0;
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
@@ -435,6 +454,14 @@ __device__ __forceinline__ void epi_select_tile(const float (&r0)[32], const flo
       const float lo4 = (jj & 2) ? ((jj & 1) ? v[3] : v[2]) : ((jj & 1) ? v[1] : v[0]);
       const float hi4 = (jj & 2) ? ((jj & 1) ? v[7] : v[6]) : ((jj & 1) ? v[5] : v[4]);
       const float x = (jj & 4) ? hi4 : lo4;
+      if constexpr (RANGE) {
+        if (cnt == cap) {
+          *cut = pos0 + 8 * q + jj;
+          thr = __int_as_float(0xFF800000);
+          gm = 0;
+          break;
+        }
+      }
       if (!REG || x < thr) {  // (REG: the threshold may have moved since the mask was made)
         buf[cnt] = ((uint64_t)__float_as_uint(x) << 32) | (uint64_t)(pos0 + 8 * q + jj);
         ++cnt;
@@ -467,6 +494,7 @@ struct TcParams {
   uint64_t* cand;          // [q_blocks][s_max][256][cap]
   int* cand_cnt;           // [q_blocks][s_max][256]   (zeroed by the host before the launch)
   float* cand_thr;         // [q_blocks][s_max][256]   final threshold (rank domain) of a piece that compacted
+  uint32_t* cand_cut;      // range mode, instead of cand_thr: position of the first dropped survivor, 0xFFFFFFFF = none
   int cap, kprime;
   int slack, hwm;          // survivors of a compaction = kprime .. kprime + slack; deferred compaction above hwm keys
   uint32_t* gthr;          // [q_pad] best threshold published per query (shared by all CTAs), 0xFF-filled
@@ -840,7 +868,9 @@ __device__ __forceinline__ void umma_tf32_2sm(uint32_t tmem_d, uint64_t desc_a, 
 
 // TcParams as for tc_scan_kernel with: pieces = the host-made table of (query block, 256-row tile range, slot) per
 // PAIR (blockIdx.x / 2; tc_ts_plan over sm_count / 2 units), s_max = candidate lists per query block = 2 x slots.
-template <int KPL>
+// RANGE: batched range queries -- every row's threshold is its query's T_q (p.gthr, filled by tc_range_threshold),
+// no compaction; a list whose buffer fills stores the position of its first dropped survivor in p.cand_cut.
+template <int KPL, bool RANGE = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
 tc_scan_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                     const __grid_constant__ CUtensorMap tmN, const __grid_constant__ CUtensorMap tmO, const TcParams p) {
@@ -1015,7 +1045,8 @@ tc_scan_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       uint64_t* buf = p.cand + (unit * TC_QB + row_in_block) * (size_t)p.cap;
       uint32_t* gthr = p.gthr + (qb * TC_QB + row_in_block);
       int cnt = 0;
-      float thr = row_valid ? __int_as_float(0x7F800000) : __int_as_float(0xFF800000);
+      float thr = !row_valid ? __int_as_float(0xFF800000) : RANGE ? f32_from_ordered(*gthr) : __int_as_float(0x7F800000);
+      uint32_t cut = 0xFFFFFFFFu;
       for (int tile = t_begin; tile < t_end; ++tile, ++ti) {
         const int b = ti & 1;
         mbar_wait(&tfull_bar[b], (ti >> 1) & 1);
@@ -1035,25 +1066,26 @@ tc_scan_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           for (int cp = 0; cp < TC_BN / 64; ++cp) {
             tmem_ld_wait();
             tmem_ld32(tcol + (uint32_t)(cp * 64 + 32), v1);
-            epi_process<KPL, false>(v0, pos_tile + cp * 64, vtile - cp * 64, buf, cnt, thr, tk_unused, p.cap, p.kprime,
-                                    p.slack, gthr, lane, ctr);
+            epi_process<KPL, false, RANGE>(v0, pos_tile + cp * 64, vtile - cp * 64, buf, cnt, thr, tk_unused, p.cap,
+                                           p.kprime, p.slack, gthr, lane, ctr, &cut);
             tmem_ld_wait();
             if (cp + 1 < TC_BN / 64) tmem_ld32(tcol + (uint32_t)(cp * 64 + 64), v0);
-            epi_process<KPL, false>(v1, pos_tile + cp * 64 + 32, vtile - cp * 64 - 32, buf, cnt, thr, tk_unused, p.cap,
-                                    p.kprime, p.slack, gthr, lane, ctr);
+            epi_process<KPL, false, RANGE>(v1, pos_tile + cp * 64 + 32, vtile - cp * 64 - 32, buf, cnt, thr, tk_unused,
+                                           p.cap, p.kprime, p.slack, gthr, lane, ctr, &cut);
           }
         }
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(b ? te_addr1 : te_addr0);  // this warp is done with the buffer (one arrival per warp)
-        if (!NB200_DBG(p.debug, 1)) {
+        if (!RANGE && !NB200_DBG(p.debug, 1)) {
           const unsigned pend = __ballot_sync(FULL, cnt > p.hwm);
           if (pend) compact_lane<KPL>(__ffs(pend) - 1, buf, cnt, thr, p.kprime, p.slack, gthr, lane);
         }
       }
       const size_t slot = unit * TC_QB + row_in_block;
       p.cand_cnt[slot] = row_valid ? cnt : 0;
-      p.cand_thr[slot] = thr;
+      if constexpr (RANGE) p.cand_cut[slot] = cut;
+      else p.cand_thr[slot] = thr;
     }
   }
 
@@ -1092,6 +1124,7 @@ struct TsParams {
   uint64_t* cand;
   int* cand_cnt;
   float* cand_thr;
+  uint32_t* cand_cut;      // range mode (see TcParams)
   int cap, kprime, slack, hwm, n_stage, use_nb, debug;
   int warm_max;            // tiles of the warm start (0 when kprime > 32: the 32 column classes bound only the 32nd best)
   int refresh_mask;        // the shared threshold is re-read every (mask + 1) tiles
@@ -1115,8 +1148,10 @@ __device__ __forceinline__ int ts_warm_tiles(int warm_max, int len) {
 }
 
 // one 32-column chunk of one row: fast path = min tree + one compare; survivors are appended to the row's
-// buffer, a full buffer is compacted warp-cooperatively first (see compact_row)
-template <int KPL, bool REG>
+// buffer, a full buffer is compacted warp-cooperatively first (see compact_row).
+// RANGE: batched range queries (fixed per-query thresholds from p.gthr, no compaction, no warm start: the host sets
+// warm_max = 0); a full buffer records its first dropped position in p.cand_cut and stops selecting.
+template <int KPL, bool REG, bool RANGE = false>
 __global__ void __launch_bounds__(TS_THREADS, 1)
 tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmN,
                   const __grid_constant__ CUtensorMap tmO, const TsParams p) {
@@ -1305,7 +1340,8 @@ tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
       uint64_t* buf = p.cand + (unit * TC_QB + h * TC_BM + row) * (size_t)p.cap;
       uint32_t* gthr = p.gthr + qrow;
       int cnt = 0;
-      float thr = row_valid ? __int_as_float(0x7F800000) : __int_as_float(0xFF800000);
+      float thr = !row_valid ? __int_as_float(0xFF800000) : RANGE ? f32_from_ordered(*gthr) : __int_as_float(0x7F800000);
+      uint32_t cut = 0xFFFFFFFFu;
       float tk[TS_RK];
 #pragma unroll
       for (int i = 0; i < TS_RK; ++i) tk[i] = __int_as_float(0x7F800000);
@@ -1373,7 +1409,8 @@ tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
         for (int j = 1; j < 32; ++j) t = fmaxf(t, gm[j]);
         if (row_valid && !NB200_DBG(p.debug, 1)) thr = publish_thr(gthr, f32_ordered(t));
       }
-      const int guard = REG ? p.cap - TS_BN - 1 : p.hwm;  // a row above this many keys sends its warp to the slow path
+      // a row above this many keys sends its warp to the slow path (RANGE: a full row has stopped selecting)
+      const int guard = RANGE ? p.cap : REG ? p.cap - TS_BN - 1 : p.hwm;
       for (int tile = t_begin; tile < t_end; ++tile) {
         uint32_t v0[32], v1[32];
         drain(v0, v1);
@@ -1417,7 +1454,7 @@ tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
             g1[q] = group_min8(r1, q);
           }
         }
-        unsigned need = __ballot_sync(FULL, cnt > p.cap - TS_BN - 1);
+        unsigned need = RANGE ? 0u : __ballot_sync(FULL, cnt > p.cap - TS_BN - 1);
         while (need) {  // about to overflow: compact at once (!REG: normally the deferred path keeps rows far from here)
           ++ctr[2];
           const int src = __ffs(need) - 1;
@@ -1429,9 +1466,9 @@ tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
         ++ctr[1];
         const uint32_t pos_tile = p.pos_base + (uint32_t)(tile * TS_BN);
         if (mm < thr || vtile < TS_BN) {
-          epi_select_tile<REG>(r0, r1, g0, g1, pos_tile, buf, cnt, thr, tk, gthr);
+          epi_select_tile<REG, RANGE>(r0, r1, g0, g1, pos_tile, buf, cnt, thr, tk, gthr, p.cap, &cut);
         }
-        if constexpr (REG) continue;
+        if constexpr (REG || RANGE) continue;
         // deferred compaction: a row past the high-water mark is compacted here, at most one row per warp and
         // tile, so the bursts (all rows of a warp fill at the same rate) are spread over the slack that every
         // tile leaves; only a row that is about to overflow is compacted at once (above)
@@ -1443,7 +1480,8 @@ tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
       }
       const size_t slot = unit * TC_QB + h * TC_BM + row;
       p.cand_cnt[slot] = row_valid ? cnt : 0;
-      p.cand_thr[slot] = thr;
+      if constexpr (RANGE) p.cand_cut[slot] = cut;
+      else p.cand_thr[slot] = thr;
     }
     if (p.counters && lane == 0) {
       for (int i = 0; i < 4; ++i) atomicAdd(p.counters + i, (unsigned long long)ctr[i]);
@@ -1892,6 +1930,14 @@ __device__ __forceinline__ float warp_sum_f(float v) {
   return v;
 }
 
+// E_q: bound on |pass-1 rank - exact rank| of one query (DESIGN.md "certificate"), shared by the kNN re-rank and the
+// range thresholds.  abs_err > 0 is an absolute bound (uint8 on the integer pipe), else eps * (2 for l2) * |q| * x_max.
+__device__ __forceinline__ float pass1_error(float abs_err, float eps_inexact, float eps_exact, bool inexact_q, int mode,
+                                             float qn2, float x_max) {
+  return abs_err > 0.f ? abs_err
+                       : (inexact_q ? eps_inexact : eps_exact) * (mode == SCAN_L2 ? 2.f : 1.f) * sqrtf(qn2) * x_max + 1e-30f;
+}
+
 __global__ void __launch_bounds__(256) tc_rerank_kernel(const RerankParams p, int items_pow2) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   uint64_t* sk = reinterpret_cast<uint64_t*>(smem_raw);          // [items_pow2] exact keys
@@ -1964,8 +2010,7 @@ __global__ void __launch_bounds__(256) tc_rerank_kernel(const RerankParams p, in
   int total = min(s_live, items_pow2);
   // pass-1 error bound of this query (same E as the certificate below)
   const bool inexact_q = p.inexact_flags[0] != 0 || p.inexact_flags[1] != 0;
-  const float E_q = p.abs_err > 0.f ? p.abs_err
-                                    : (inexact_q ? p.eps_inexact : p.eps_exact) * (p.mode == SCAN_L2 ? 2.f : 1.f) * sqrtf(qn2) * p.x_max + 1e-30f;
+  const float E_q = pass1_error(p.abs_err, p.eps_inexact, p.eps_exact, inexact_q, p.mode, qn2, p.x_max);
   {
     // Second filter.  Let a_k be the k-th smallest PASS-1 rank among the live keys.  The k keys at or below it
     // have exact rank <= a_k + E, so the true k-th best exact rank is <= a_k + E and every true neighbour has
@@ -2185,6 +2230,51 @@ __global__ void __launch_bounds__(256) tc_rerank_kernel(const RerankParams p, in
              s_live, total, p2e, items_pow2, minthr, worst, qn2, p.n_split, s_cnt[0]);
     }
   }
+}
+
+// ---------------------------------------------------------------- batched range queries: radius -> threshold
+// One warp per query.  T_q is the radius in the rank domain of pass 1 (see the header of this file), widened so that
+// every row whose distance by the verification formula (range_scan.cu: range_row_dist) is <= r has pass-1 rank < T_q
+// (DESIGN.md "K5b"): E_q of the re-rank's certificate, plus rel = (D + 16) 2^-22 -- about four times the first-order
+// fp32 error of the verification sums and of |q|^2 -- on every term, evaluated in double and rounded up.
+__global__ void tc_range_threshold_kernel(const float* __restrict__ q, int nq, int row_words, int mode, int take_sqrt,
+                                          const float* __restrict__ radii, float x_max, float eps_inexact,
+                                          float eps_exact, int db_inexact, uint32_t* __restrict__ gthr) {
+  const int qi = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (qi >= nq) return;
+  const float* qv = q + (size_t)qi * row_words;
+  float s = 0.f;
+  unsigned bad = 0;
+  for (int c = lane; c < row_words; c += 32) {
+    const float v = qv[c];
+    s = fmaf(v, v, s);
+    bad |= __float_as_uint(v) & 0x1FFFu;  // not TF32-exact (as the scan kernels test it)
+  }
+  s = warp_sum_f(s);
+  bad = __reduce_or_sync(FULL, bad);
+  if (lane != 0) return;
+  const float E = pass1_error(0.f, eps_inexact, eps_exact, bad != 0 || db_inexact != 0, mode, s, x_max);
+  const double r = radii[qi], qn2 = s, qn = sqrt(qn2), xm = x_max;
+  const double rel = (row_words + 16) * 2.384185791015625e-07;
+  double t;
+  if (mode == SCAN_L2) {  // d^2 <= r^2 (l2sqr: d <= r)  <=>  |x|^2 - 2 q.x <= r^2 - |q|^2
+    const double r2 = take_sqrt ? r * r : r;
+    t = r2 - qn2 + rel * (r2 + qn2 + xm * xm);
+  } else if (mode == SCAN_NEGDOT) {  // -q.x <= r
+    t = r + 2.0 * rel * qn * xm;
+  } else if (s < 1e-30f) {
+    // cosine family, a query of (almost) zero norm: the verification formula takes nsp = 0 when |q|^2 < 2 FLT_MIN
+    // (d = 1, or pi / 2) whatever its pass-1 rank -q.x/|x| is, so no rank threshold is valid -- admit every row
+    // (1e-30 leaves a margin of ~2^33 over 2 FLT_MIN: the fp32 |q|^2 of the two kernels cannot straddle the test)
+    t = INFINITY;
+  } else if (mode == SCAN_COSINE) {  // 1 - nsp <= r  <=>  -|q| nsp <= -|q| (1 - r); r >= 2 admits every row
+    t = r >= 2.0 ? INFINITY : qn * (r - 1.0) + 4.0 * rel * qn;
+  } else {  // SCAN_ANGULAR: acos(nsp) <= r  <=>  nsp >= cos r (acosf is within 2 ulp: < 5e-7 below pi); r >= pi admits all
+    const double ra = r + 1e-6;
+    t = ra >= 3.14159265358979323846 ? INFINITY : -qn * cos(ra) + 4.0 * rel * qn;
+  }
+  // rank < T_q is strict: one more ulp above the rounded-up bound
+  gthr[qi] = f32_ordered(nextafterf(__double2float_ru(t + (double)E), INFINITY));
 }
 
 // ---------------------------------------------------------------- operand preparation
@@ -2614,7 +2704,7 @@ int tc_pair_block_points() { return TP_BN; }
 cudaError_t launch_tc_scan_pair(const float* qa, size_t q_pad, const float* dbB, size_t n_pad, const float* nblock,
                                 const float* ones, int n, int nq, int row_words, int k, uint32_t pos_base, int n_pairs,
                                 const int* d_pieces, int s_max, int kprime, uint64_t* cand, int* cand_cnt,
-                                float* cand_thr, uint32_t* gthr, cudaStream_t stream) {
+                                float* cand_thr, uint32_t* gthr, cudaStream_t stream, uint32_t* range_cut) {
   if (n <= 0 || nq <= 0) return cudaSuccess;
   if (row_words % TC_KB) return cudaErrorInvalidValue;
   CUtensorMap tmA, tmB, tmN, tmO;
@@ -2647,6 +2737,8 @@ cudaError_t launch_tc_scan_pair(const float* qa, size_t q_pad, const float* dbB,
   p.slack = std::max(8, p.kprime / 4);
   p.hwm = std::min(p.cap / 2, std::max(64, 2 * p.kprime));
   p.gthr = gthr;
+  p.cand_cut = range_cut;
+  if (range_cut) p.cap = tc_range_cap();
   p.use_nb = use_nb ? 1 : 0;
   {
     const char* dbg = nb200_env("NB200_TC_DEBUG");
@@ -2660,14 +2752,16 @@ cudaError_t launch_tc_scan_pair(const float* qa, size_t q_pad, const float* dbB,
   if (p.n_stage > 8) p.n_stage = 8;
   const size_t smem = 1024 + (size_t)ones_bytes + (size_t)p.n_stage * stage_bytes + (2 * 8 + 12) * 8 + 16;
   cudaError_t e;
-#define NB_TP(KPL)                                                                                            \
-  e = cudaFuncSetAttribute(tc_scan_pair_kernel<KPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-  if (e != cudaSuccess) return e;                                                                             \
-  tc_scan_pair_kernel<KPL><<<2 * n_pairs, TC_THREADS, smem, stream>>>(tmA, tmB, tmN, tmO, p);
-  if (p.cap == 256) {
-    NB_TP(8);
+#define NB_TP(KPL, RANGE)                                                                                             \
+  e = cudaFuncSetAttribute(tc_scan_pair_kernel<KPL, RANGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+  if (e != cudaSuccess) return e;                                                                                     \
+  tc_scan_pair_kernel<KPL, RANGE><<<2 * n_pairs, TC_THREADS, smem, stream>>>(tmA, tmB, tmN, tmO, p);
+  if (range_cut) {
+    NB_TP(8, true);
+  } else if (p.cap == 256) {
+    NB_TP(8, false);
   } else {
-    NB_TP(16);
+    NB_TP(16, false);
   }
 #undef NB_TP
   e = cudaGetLastError();
@@ -2781,7 +2875,8 @@ void tc_ts_plan(int nq, int n, int k, int sm_count, std::vector<int>* table, int
 cudaError_t launch_tc_scan_ts(const float* q, const float* dbB, size_t n_pad, const float* nblock, const float* ones,
                               int n, int nq, int row_words, int k, int kprime, float scale, uint32_t pos_base,
                               int n_cta, int s_max, const int* d_pieces, uint64_t* cand, int* cand_cnt,
-                              float* cand_thr, uint32_t* gthr, int* inexact_flag, cudaStream_t stream) {
+                              float* cand_thr, uint32_t* gthr, int* inexact_flag, cudaStream_t stream,
+                              uint32_t* range_cut) {
   if (n <= 0 || nq <= 0) return cudaSuccess;
   if (!tc_ts_supported(row_words)) return cudaErrorInvalidValue;
   CUtensorMap tmB, tmN, tmO;
@@ -2817,6 +2912,11 @@ cudaError_t launch_tc_scan_ts(const float* q, const float* dbB, size_t n_pad, co
   if (const char* e = nb200_env("NB200_TC_WARM")) p.warm_max = p.kprime <= 32 ? std::max(0, atoi(e)) : 0;
   if (const char* e = nb200_env("NB200_TC_REFRESH")) p.refresh_mask = std::max(0, atoi(e));
   p.gthr = gthr;
+  p.cand_cut = range_cut;
+  if (range_cut) {  // range mode: fixed thresholds, so no warm start
+    p.cap = tc_range_cap();
+    p.warm_max = 0;
+  }
   p.use_nb = use_nb ? 1 : 0;
   {
     const char* dbg = nb200_env("NB200_TC_DEBUG");
@@ -2854,25 +2954,27 @@ cudaError_t launch_tc_scan_ts(const float* q, const float* dbB, size_t n_pad, co
   if (p.n_stage < 2) return cudaErrorInvalidValue;
   const size_t smem = 1024 + (size_t)ones_bytes + (size_t)p.n_stage * stage_bytes + (2 * 8 + 12) * 8 + 16;
   cudaError_t e;
-#define NB_TS(KPL, REG)                                                                                           \
-  e = cudaFuncSetAttribute(tc_scan_ts_kernel<KPL, REG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);  \
-  if (e != cudaSuccess) return e;                                                                                 \
-  tc_scan_ts_kernel<KPL, REG><<<n_cta, TS_THREADS, smem, stream>>>(tmB, tmN, tmO, p);
+#define NB_TS(KPL, REG, RANGE)                                                                                          \
+  e = cudaFuncSetAttribute(tc_scan_ts_kernel<KPL, REG, RANGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+  if (e != cudaSuccess) return e;                                                                                       \
+  tc_scan_ts_kernel<KPL, REG, RANGE><<<n_cta, TS_THREADS, smem, stream>>>(tmB, tmN, tmO, p);
   static const bool no_reg = [] {
     const char* e2 = nb200_env("NB200_TC_NO_REG");
     return e2 && e2[0] == '1';
   }();
   // register list (16 ranks): k <= 12 leaves the certificate a margin of >= 4 ranks; a margin raised by the
   // engine (certificates failed on inexact data) selects the buffer path with its larger k'
-  if (k + 4 <= TS_RK && kprime <= k + 6 && p.cap == 256 && !no_reg) {
+  if (range_cut) {
+    NB_TS(8, false, true);
+  } else if (k + 4 <= TS_RK && kprime <= k + 6 && p.cap == 256 && !no_reg) {
     p.kprime = TS_RK;  // the register list always holds 16
     p.slack = 8;
     if (!nb200_env("NB200_TC_WARM")) p.warm_max = 0;  // exact thresholds make the cold start cheaper than the re-scan
-    NB_TS(8, true);
+    NB_TS(8, true, false);
   } else if (p.cap == 256) {
-    NB_TS(8, false);
+    NB_TS(8, false, false);
   } else {
-    NB_TS(16, false);
+    NB_TS(16, false, false);
   }
 #undef NB_TS
   e = cudaGetLastError();
@@ -2880,6 +2982,25 @@ cudaError_t launch_tc_scan_ts(const float* q, const float* dbB, size_t n_pad, co
     fprintf(stderr, "nmslib_b200: tc_scan_ts launch (grid %d, smem %zu, stages %d) failed: %s\n", n_cta, smem,
             p.n_stage, cudaGetErrorString(e));
   return e;
+}
+
+// Error model of pass 1 (DESIGN.md "certificate"): TF32 operands are fp32 with the low 13 mantissa
+// bits dropped (relative 2^-10 each when truncated), products exact, fp32 accumulation over D terms.
+static void pass1_eps(int row_words, float* eps_exact, float* eps_inexact) {
+  *eps_exact = (float)row_words * 2.384185791015625e-07f;         // D * 2^-22  (accumulation only)
+  *eps_inexact = 2.0f * 0.0009765625f * 1.01f + *eps_exact;       // 2 * 2^-10 + accumulation
+}
+
+int tc_range_cap() { return 256; }
+
+cudaError_t launch_tc_range_threshold(const float* q, int nq, int row_words, int mode, int take_sqrt, const float* radii,
+                                      float x_max, int db_inexact, uint32_t* gthr, cudaStream_t stream) {
+  if (nq <= 0) return cudaSuccess;
+  float eps_exact, eps_inexact;
+  pass1_eps(row_words, &eps_exact, &eps_inexact);
+  tc_range_threshold_kernel<<<(nq + 7) / 8, 256, 0, stream>>>(q, nq, row_words, mode, take_sqrt, radii, x_max,
+                                                              eps_inexact, eps_exact, db_inexact, gthr);
+  return cudaGetLastError();
 }
 
 // live keys the re-rank's sort buffer must hold for a query with n_lists candidate lists of `cap` keys
@@ -2926,11 +3047,7 @@ cudaError_t launch_tc_rerank(const float* db, const float* queries, const float*
   p.cand = cand;
   p.cand_cnt = cand_cnt;
   p.cand_thr = cand_thr;
-  // Error model of pass 1 (DESIGN.md "certificate"): TF32 operands are fp32 with the low 13 mantissa
-  // bits dropped (relative 2^-10 each when truncated), products exact, fp32 accumulation over D terms.
-  const float dterms = (float)row_words;
-  p.eps_exact = dterms * 2.384185791015625e-07f;                    // D * 2^-22  (accumulation only)
-  p.eps_inexact = 2.0f * 0.0009765625f * 1.01f + p.eps_exact;       // 2 * 2^-10 + accumulation
+  pass1_eps(row_words, &p.eps_exact, &p.eps_inexact);
   if (eps_override > 0.f) p.eps_exact = p.eps_inexact = eps_override;  // (split operands: see Engine::enable_split)
   p.x_max = x_max;
   p.inexact_flags = inexact_flags;

@@ -391,6 +391,54 @@ Status ShardGroup::knn_host(Engine* host, const void* queries, size_t nq, size_t
   return Status::OK();
 }
 
+// Shards hold contiguous position ranges in shard order, so a query's global answer (rows within the radius in
+// position order, truncated to the capacity) is the shards' answers -- each truncated to the capacity -- concatenated
+// and truncated: a host step, no device exchange.
+Status ShardGroup::range_host(Engine* host, const void* queries, size_t nq, size_t elem_count, const double* radii,
+                              const size_t* caps, int32_t* const* ids, float* const* dists, size_t* sizes) {
+  Impl& m = *impl_;
+  for (size_t i = 0; i < nq; ++i) sizes[i] = 0;
+  if (!host->built()) return Status::Err(8, "Index not built");
+  if (m.method != METHOD_SEQ)
+    return Status::Err(5, "Range query not supported by method: Range search is not supported!");
+  // (the order of Engine::range_batch_host: no device is an error even for an empty index)
+  if (!device_available()) return Status::Err(kErrQuery, "no CUDA device available (there is no CPU fallback)");
+  if (host->size() == 0 || nq == 0) return Status::OK();
+  Status s = prepare(host, 0, 0);
+  if (!s.ok()) return s;
+  const size_t G = (size_t)m.active;
+  std::vector<size_t> off(nq + 1, 0);
+  for (size_t i = 0; i < nq; ++i) off[i + 1] = off[i] + std::min(caps[i], host->size());
+  std::vector<std::vector<int32_t>> sid(G, std::vector<int32_t>(off[nq]));
+  std::vector<std::vector<float>> sd(G, std::vector<float>(off[nq]));
+  std::vector<std::vector<size_t>> ssz(G, std::vector<size_t>(nq));
+  s = m.run_all([&](int g) -> Status {
+    std::vector<int32_t*> pi(nq);
+    std::vector<float*> pd(nq);
+    std::vector<size_t> c(nq);
+    for (size_t i = 0; i < nq; ++i) {
+      pi[i] = sid[g].data() + off[i];
+      pd[i] = sd[g].data() + off[i];
+      c[i] = off[i + 1] - off[i];
+    }
+    std::lock_guard<std::mutex> lock(m.shards[g]->mutex());
+    return m.shards[g]->range_batch_host(queries, nq, elem_count, radii, c.data(), pi.data(), pd.data(), ssz[g].data());
+  });
+  if (!s.ok()) return s;
+  for (size_t i = 0; i < nq; ++i) {
+    size_t at = 0;
+    for (size_t g = 0; g < G && at < caps[i]; ++g) {
+      const size_t take = std::min(ssz[g][i], caps[i] - at);
+      memcpy(ids[i] + at, sid[g].data() + off[i], take * 4);
+      memcpy(dists[i] + at, sd[g].data() + off[i], take * 4);
+      at += take;
+    }
+    sizes[i] = at;
+  }
+  m.stats.queries += nq;
+  return Status::OK();
+}
+
 Stats ShardGroup::stats() {
   Stats out = impl_->stats;
   for (auto& e : impl_->shards) {
@@ -402,6 +450,8 @@ Stats ShardGroup::stats() {
     out.hnsw_expansions += s.hnsw_expansions;
     out.fallback_queries += s.fallback_queries;
     out.split_queries += s.split_queries;
+    out.range_tc_queries += s.range_tc_queries;
+    out.range_fallback_queries += s.range_fallback_queries;
     out.device_bytes += s.device_bytes;
     out.uploaded_rows += s.uploaded_rows;
     out.last_scan_ms = std::max(out.last_scan_ms, s.last_scan_ms);

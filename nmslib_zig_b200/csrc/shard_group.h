@@ -22,6 +22,9 @@ class ShardGroup {
   // host in / host out over all shards: ids / dists / counts point at the group's pinned result arrays
   Status knn_host(Engine* host_store, const void* queries, size_t nq, size_t elem_count, size_t k, const int32_t** ids,
                   const float** dists, const int32_t** counts);
+  // batched range queries (seq_search): every shard answers over its rows, the lists are concatenated in shard order
+  Status range_host(Engine* host_store, const void* queries, size_t nq, size_t elem_count, const double* radii,
+                    const size_t* caps, int32_t* const* ids, float* const* dists, size_t* sizes);
   Status prepare(Engine* host_store, size_t nq, size_t k);
   Stats stats();
 

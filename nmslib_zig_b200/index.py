@@ -67,7 +67,8 @@ class Stats(C.Structure):
                 ("scan_ms_sum", C.c_double), ("scan_count", C.c_uint64), ("build_total_ms", C.c_double),
                 ("build_scan_ms", C.c_double), ("build_select_ms", C.c_double), ("build_link_ms", C.c_double),
                 ("build_batches", C.c_uint64), ("build_prunes", C.c_uint64), ("split_queries", C.c_uint64),
-                ("u8_imma", C.c_uint64), ("uploaded_rows", C.c_uint64)]
+                ("u8_imma", C.c_uint64), ("uploaded_rows", C.c_uint64), ("range_tc_queries", C.c_uint64),
+                ("range_fallback_queries", C.c_uint64)]
 
 
 # every symbol include/nmslib_b200.h declares (the CPU-side test checks this list against the header)
@@ -88,6 +89,7 @@ EXT_SYMBOLS = [
     "nmslib_b200_prepare", "nmslib_b200_knn_device", "nmslib_b200_merge_topk", "nmslib_b200_get_stats",
     "nmslib_b200_version", "nmslib_b200_scan_plan", "nmslib_b200_scan_plan_pairs", "nmslib_b200_set_option",
     "nmslib_b200_shard_export", "nmslib_b200_shard_connect", "nmslib_b200_shard_disconnect",
+    "nmslib_b200_range_query_batch",
 ]
 
 _lib = None
@@ -181,6 +183,7 @@ def lib() -> C.CDLL:
         "nmslib_b200_shard_export": (C.c_int, [vp, sz, sz, vp]),
         "nmslib_b200_shard_connect": (C.c_int, [vp, C.c_int, C.c_int, vp]),
         "nmslib_b200_shard_disconnect": (C.c_int, [vp]),
+        "nmslib_b200_range_query_batch": (C.c_int, [vp, vp, sz, sz, C.POINTER(C.c_double), C.POINTER(Result)]),
         "nmslib_b200_scan_plan": (sz, [sz, sz, sz, C.c_int, vp, sz, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
         "nmslib_b200_scan_plan_pairs": (sz, [sz, sz, sz, C.c_int, vp, sz, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     }
@@ -413,6 +416,39 @@ class Index:
         res = Result(ids.ctypes.data_as(C.POINTER(C.c_int32)), dists.ctypes.data_as(C.POINTER(C.c_float)), 0, cap)
         _check(L.nmslib_range_query_fill(self.handle, q.ctypes.data, q.size, radius, C.byref(res), 0))
         return QueryResult(ids[: res.size], dists[: res.size])
+
+    def rangeQueryBatch(self, queries, radius, capacity=128) -> BatchResult:
+        """nmslib_b200 extension: ONE nmslib_b200_range_query_batch call for [Q, dim] queries.  `radius` and
+        `capacity` are scalars or [Q] arrays.  Every row is what rangeQuery returns for that query (objects within
+        the radius in position order, truncated to the capacity), padded to the largest capacity with id -1 /
+        distance +inf; `sizes` holds the counts."""
+        L = lib()
+        if not self.built:
+            self.buildIndex(None, False)
+        q = np.ascontiguousarray(queries, self._elem_dtype())
+        if q.ndim != 2:
+            raise NmslibError(2, "queries must be [Q, dim]")
+        nq, dim = q.shape
+        radii = np.ascontiguousarray(np.broadcast_to(np.asarray(radius, np.float64), (nq,)))
+        caps = np.broadcast_to(np.asarray(capacity, np.int64), (nq,))
+        if nq and caps.min() < 0:
+            raise NmslibError(2, "negative capacity")
+        width = int(caps.max()) if nq else 0
+        ids = np.full((nq, width), -1, np.int32)
+        dists = np.full((nq, width), np.inf, np.float32)
+        if nq == 0:
+            return BatchResult(ids, dists, np.empty(0, np.int64))
+        results = (Result * nq)()
+        tbl = np.frombuffer(results, dtype=np.uint64).reshape(nq, 4)
+        row = np.arange(nq, dtype=np.uint64) * np.uint64(4 * width)
+        tbl[:, 0] = row + np.uint64(ids.ctypes.data)
+        tbl[:, 1] = row + np.uint64(dists.ctypes.data)
+        tbl[:, 2] = 0
+        tbl[:, 3] = caps.astype(np.uint64)
+        _check(L.nmslib_b200_range_query_batch(self.handle, q.ctypes.data, nq, dim,
+                                               radii.ctypes.data_as(C.POINTER(C.c_double)), results))
+        sizes = tbl[:, 2].astype(np.int64)
+        return BatchResult(ids, dists, sizes)
 
     # -- data access ---------------------------------------------------------------------
     def getDistance(self, pos1: int, pos2: int) -> float:

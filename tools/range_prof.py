@@ -1,0 +1,122 @@
+"""Timing of the batched range queries (nmslib_b200_range_query_batch, K5b) against the per-query range path.
+
+usage: range_prof.py [--n N] [--nq Q] [--sample S] [--out FILE]
+
+Two shapes: n x 128 l2 (TS kernel) and n x 768 cosinesimil (pair kernel), Q queries each, radius at the 10th and
+at the 100th neighbour of every query, capacity 128.  For each it reports the batch wall time (host in / host out),
+the pass-1 kernel time (CUDA events, stats.last_scan_ms) and its TFLOP/s (2 Q N D) against the 1 108 TFLOP/s TF32
+stream peak DESIGN.md uses, the threshold and verification kernel times (torch.profiler, a separate run), the
+fallback count, and the per-query rangeQuery time over S queries.  Prints the GPU name and power limit first.
+Defaults: n = 1 000 000, Q = 10 000, S = 200."""
+import argparse
+import json
+import subprocess
+import sys
+import time
+from pathlib import Path
+
+import numpy as np
+
+sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
+import nmslib_zig_b200 as nb  # noqa: E402
+from nmslib_zig_b200 import synth  # noqa: E402
+
+TF32_PEAK = 1108.0  # TFLOP/s, DESIGN.md (tools/tc_peak.cu stream peak)
+
+
+def gpu_info():
+    import torch
+    name = torch.cuda.get_device_name(0)
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+    except Exception as e:  # (reported, not guessed)
+        out = f"unavailable ({e})"
+    return {"gpu": name, "power_limit_and_max_sm_clock": out}
+
+
+def kernel_times(fn):
+    """device time per kernel name (ms) of one call of fn, from torch.profiler with CUDA activities"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    out = {}
+    for ev in prof.events():
+        t = getattr(ev, "device_time_total", 0)
+        for key in ("tc_range_threshold", "tc_scan_ts", "tc_scan_pair", "range_verify", "range_dist", "range_collect"):
+            if key in ev.name:
+                out[key] = out.get(key, 0.0) + t / 1e3
+    return out
+
+
+def run_shape(space, n, dim, nq, sample, emit):
+    data = synth.uniform(n, dim, 3) - 0.3
+    q = synth.uniform(nq, dim, 4) - 0.3
+    idx = nb.Index(space, None, "seq_search")
+    idx.addDenseBatch(data)
+    idx.buildIndex()
+    if not nb.device_available():  # (a CPU rehearsal gets this far: arguments, data, index construction)
+        raise SystemExit(f"range_prof.py: {space} {n}x{dim} index built; the measurements need a CUDA device, none is visible")
+    kd = idx.knnQueryBatch(q, 100).distances
+    for nth in (10, 100):
+        radii = kd[:, nth - 1].astype(np.float64)
+        idx.rangeQueryBatch(q, radii, 128)                      # warm-up (module load, scratch allocation)
+        walls, scans = [], []
+        for _ in range(3):
+            st0 = idx.stats()
+            t0 = time.perf_counter()
+            r = idx.rangeQueryBatch(q, radii, 128)
+            walls.append((time.perf_counter() - t0) * 1e3)
+            st = idx.stats()
+            scans.append(st["last_scan_ms"])
+        fb = st["range_fallback_queries"] - st0["range_fallback_queries"]
+        tcq = st["range_tc_queries"] - st0["range_tc_queries"]
+        ktimes = kernel_times(lambda: idx.rangeQueryBatch(q, radii, 128))
+        pick = np.linspace(0, nq - 1, sample).astype(int)
+        idx.rangeQuery(q[pick[0]], float(radii[pick[0]]), capacity=128)
+        t0 = time.perf_counter()
+        for i in pick:
+            idx.rangeQuery(q[i], float(radii[i]), capacity=128)
+        per_q = (time.perf_counter() - t0) * 1e3 / len(pick)
+        pass1 = min(scans)
+        flop = 2.0 * nq * n * dim
+        rec = {"space": space, "n": n, "dim": dim, "nq": nq, "radius_at_neighbour": nth, "capacity": 128,
+               "batch_wall_ms": round(min(walls), 3), "pass1_ms": round(pass1, 4),
+               "pass1_tflops": round(flop / (pass1 * 1e-3) / 1e12, 1) if pass1 > 0 else None,
+               "pass1_share_of_tf32_peak": round(flop / (pass1 * 1e-3) / 1e12 / TF32_PEAK, 3) if pass1 > 0 else None,
+               "kernel_ms_profiler": {k: round(v, 4) for k, v in ktimes.items()},
+               "tc_queries": int(tcq), "fallback_queries": int(fb),
+               "mean_hits": round(float(r.sizes.mean()), 2),
+               "single_query_ms": round(per_q, 4), "single_query_x_Q_ms": round(per_q * nq, 1),
+               "speedup_vs_single": round(per_q * nq / min(walls), 1)}
+        emit(rec)
+    idx.deinit()
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--n", type=int, default=1_000_000)
+    ap.add_argument("--nq", type=int, default=10_000)
+    ap.add_argument("--sample", type=int, default=200)
+    ap.add_argument("--out", default=None)
+    a = ap.parse_args()
+    lines = []
+
+    def emit(rec):
+        s = json.dumps(rec)
+        print(s, flush=True)
+        lines.append(s)
+
+    if nb.device_available():
+        emit(gpu_info())
+    run_shape("l2", a.n, 128, a.nq, a.sample, emit)
+    run_shape("cosinesimil", a.n, 768, a.nq, a.sample, emit)
+    if a.out:
+        with open(a.out, "w") as f:
+            f.write("\n".join(lines) + "\n")
+
+
+if __name__ == "__main__":
+    main()
