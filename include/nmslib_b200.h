@@ -283,7 +283,7 @@ typedef struct {
   uint64_t u8_imma;          /* 1: uint8 rows are scanned on the integer tensor pipe (tcgen05.mma.kind::i8), 0: widened to TF32 */
   uint64_t uploaded_rows;    /* rows copied host -> device so far (an append uploads only the new rows) */
   /* nmslib_b200_range_query_batch (b200_devices indexes: counted once per shard) */
-  uint64_t range_tc_queries;       /* range queries whose answer came from the tensor-core pass */
+  uint64_t range_tc_queries;       /* range queries whose answer came from the tensor-core pass (uint8 included) */
   uint64_t range_fallback_queries; /* range queries re-run by the per-query exact scan (tensor-core pass uncertified) */
 } nmslib_b200_stats_t;
 nmslib_error_t nmslib_b200_get_stats(nmslib_index_handle_t index, nmslib_b200_stats_t* out);
@@ -298,10 +298,10 @@ nmslib_error_t nmslib_b200_get_stats(nmslib_index_handle_t index, nmslib_b200_st
  * any work; a query length that does not match the index -> QUERY_EXECUTION_FAILED; hnsw -> SPACE_INCOMPATIBLE
  * (the reference has no range search over hnsw); an index that is not built -> INDEX_BUILD_FAILED, as for
  * nmslib_range_query_fill.  An empty index returns size 0 everywhere.
- * l2, l2sqr, cosinesimil, negdotprod and angulardist run as one tensor-core pass over the rows for the whole batch
- * (a threshold per query, verified with the per-query scan's own distance code); l1, linf, uint8 indexes
- * (l2sqr_sift: the integer-pipe kernel has no range mode yet), force_exact and, under option tc_pair=0, rows of more
- * than 128 floats use the per-query exact scan, as does
+ * l2, l2sqr, cosinesimil, negdotprod, angulardist and l2sqr_sift run as one tensor-core pass over the rows for the
+ * whole batch (a threshold per query, verified with the per-query scan's own distance code; uint8 byte rows on the
+ * integer tensor pipe with an exact integer threshold, widened uint8 rows on the TF32 pass); l1, linf, force_exact
+ * and, under option tc_pair=0, rows of more than 128 floats use the per-query exact scan, as does
  * any query the tensor-core pass cannot certify (nmslib_b200_stats_t counts both).  A b200_devices index answers
  * over every shard and concatenates the shards' lists in position order. */
 nmslib_error_t nmslib_b200_range_query_batch(nmslib_index_handle_t index, const void* queries,

@@ -1418,10 +1418,11 @@ Status Engine::range_host(const void* query, size_t elem_count, double radius, s
 }
 
 // Batched range queries (K5b, DESIGN.md): the answer of range_host for every query, one device submission per chunk.
-// Float spaces with a dot-product form run on the tensor cores: radius -> pass-1 threshold T_q, the TS / pair scan
-// in range mode (survivors of rank < T_q in position order, a position cut where a list fills), verification of the
-// candidates with the per-query scan's own distance code.  l1 / linf / uint8 / force_exact, and every query the
-// tensor-core pass cannot certify, take the per-query exact scan (launch_range_scan) inside the same submission.
+// Float spaces with a dot-product form and uint8 run on the tensor cores: radius -> pass-1 threshold T_q (uint8 byte
+// rows: an integer accumulator threshold), the TS / pair / u8 scan in range mode (survivors beating the threshold in
+// position order, a position cut where a list fills), verification of the candidates with the per-query scan's own
+// distance code.  l1 / linf / force_exact, and every query the tensor-core pass cannot certify, take the per-query
+// exact scan (launch_range_scan) inside the same submission.
 // Outputs are staged in CSR form (min(capacity, n) slots per query); a batch whose staging would exceed
 // kRangeStageBytes runs in query chunks.
 namespace {
@@ -1470,12 +1471,15 @@ Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, co
   const int mode = range_mode();
   const int take_sqrt = space_ == SPACE_L2 ? 1 : 0;
   // the tensor-core pass needs the TS kernel (rows <= 128 floats) or the pair kernel; with option tc_pair=0 longer
-  // rows take the per-query exact scan like l1 / linf (not counted as fallbacks: no tensor-core pass was made)
-  const bool ts = tc_ts_supported(row_words_);
+  // rows take the per-query exact scan like l1 / linf (not counted as fallbacks: no tensor-core pass was made).
+  // uint8: byte rows run the integer-pipe kernel (tc_scan_u8_kernel) over the TS piece table; widened rows (option
+  // u8_imma=0, or norms beyond the digit block) are exact integers in fp32 and take the TS kernel like l2sqr
+  const bool u8 = u8_imma_;  // (never with force_exact)
+  const bool ts = u8 || tc_ts_supported(row_words_);
   const bool pair = !ts && tc_pair_enabled() && sm_count_ >= 2;
-  const bool tc = !force_exact_ && !is_u8_ && (ts || pair) &&
-                  (space_ == SPACE_L2 || space_ == SPACE_L2SQR || space_ == SPACE_COSINE || space_ == SPACE_NEGDOT ||
-                   space_ == SPACE_ANGULAR);
+  const bool tc = !force_exact_ && (ts || pair) &&
+                  (u8 || u8_widened() || space_ == SPACE_L2 || space_ == SPACE_L2SQR || space_ == SPACE_COSINE ||
+                   space_ == SPACE_NEGDOT || space_ == SPACE_ANGULAR);
   Status s = stage_queries_device(queries, false, nq, elem_count, stream_);
   if (!s.ok()) return s;
   // per-query parameters: radii [nq] f32 | caps [nq] i32 | CSR offsets [nq] i64; outputs: counts [nq] | fallback
@@ -1540,9 +1544,12 @@ Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, co
     if (!(s = check_cuda(cudaMemsetAsync(d_fb_cnt, 0, 4, stream_), "memset(range fb count)")).ok()) return s;
     const int tmode = space_ == SPACE_COSINE ? SCAN_COSINE : space_ == SPACE_ANGULAR ? SCAN_ANGULAR
                       : space_ == SPACE_NEGDOT ? SCAN_NEGDOT : SCAN_L2;
-    s = check_cuda(launch_tc_range_threshold(d_q_.as<float>(), (int)nq, row_words_, tmode, take_sqrt, d_radii, x_max_,
-                                             db_inexact_ ? 1 : 0, d_rthr_.as<uint32_t>(), stream_),
-                   "tc_range_threshold");
+    s = u8 ? check_cuda(launch_tc_range_threshold_u8(d_q_.as<uint8_t>(), (int)nq, d_radii, u8_m_half_,
+                                                     d_rthr_.as<uint32_t>(), stream_),
+                        "tc_range_threshold_u8")
+           : check_cuda(launch_tc_range_threshold(d_q_.as<float>(), (int)nq, row_words_, tmode, take_sqrt, d_radii,
+                                                  x_max_, db_inexact_ ? 1 : 0, d_rthr_.as<uint32_t>(), stream_),
+                        "tc_range_threshold");
     if (!s.ok()) return s;
     // pass 1 on the plain operands (never the split copy): the threshold's error band covers TF32-inexact data
     const bool cosf = tmode == SCAN_COSINE || tmode == SCAN_ANGULAR;
@@ -1558,15 +1565,19 @@ Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, co
       ++stats_.kernel_launches;
     }
     scan_begin(stream_);
-    s = check_cuda(ts ? launch_tc_scan_ts(d_q_.as<float>(), dbB, n_pad, nbp, d_ones_.as<float>(), (int)n_dev_, (int)nq,
-                                          row_words_, 1, 0, scale, pos_base_, n_cta, s_max, d_rplan_.as<int>(),
-                                          d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), nullptr, d_rthr_.as<uint32_t>(),
-                                          d_flags_.as<int>() + 1, stream_, d_rcut_.as<uint32_t>())
-                      : launch_tc_scan_pair(d_qa_.as<float>(), q_pad, dbB, n_pad, nbp, d_ones_.as<float>(), (int)n_dev_,
-                                            (int)nq, row_words_, 1, pos_base_, n_cta, d_rplan_.as<int>(), s_max, 0,
+    s = check_cuda(u8   ? launch_tc_scan_u8(d_q_.as<uint8_t>(), d_db_.as<uint8_t>(), d_digits_.as<uint8_t>(), n_pad,
+                                            (int)n_dev_, (int)nq, 1, 0, u8_m_half_, pos_base_, n_cta, s_max,
+                                            d_rplan_.as<int>(), d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), nullptr,
+                                            d_rthr_.as<uint32_t>(), stream_, d_rcut_.as<uint32_t>())
+                   : ts ? launch_tc_scan_ts(d_q_.as<float>(), dbB, n_pad, nbp, d_ones_.as<float>(), (int)n_dev_, (int)nq,
+                                            row_words_, 1, 0, scale, pos_base_, n_cta, s_max, d_rplan_.as<int>(),
                                             d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), nullptr, d_rthr_.as<uint32_t>(),
-                                            stream_, d_rcut_.as<uint32_t>()),
-                   ts ? "tc_scan_ts(range)" : "tc_scan_pair(range)");
+                                            d_flags_.as<int>() + 1, stream_, d_rcut_.as<uint32_t>())
+                        : launch_tc_scan_pair(d_qa_.as<float>(), q_pad, dbB, n_pad, nbp, d_ones_.as<float>(), (int)n_dev_,
+                                              (int)nq, row_words_, 1, pos_base_, n_cta, d_rplan_.as<int>(), s_max, 0,
+                                              d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), nullptr, d_rthr_.as<uint32_t>(),
+                                              stream_, d_rcut_.as<uint32_t>()),
+                   u8 ? "tc_scan_u8(range)" : ts ? "tc_scan_ts(range)" : "tc_scan_pair(range)");
     scan_end(stream_);
     if (!s.ok()) return s;
     s = check_cuda(launch_range_verify(d_db_.as<float>(), d_q_.as<float>(), d_ids_.as<int32_t>(), row_words_, mode,

@@ -147,7 +147,12 @@ cudaError_t launch_u8_max_norm(const int* norm2, int n, int* d_out, cudaStream_t
 cudaError_t launch_u8_norm_digits(const int* norm2, int n, int n_pad, int m_half, uint8_t* out, cudaStream_t stream);
 cudaError_t launch_tc_scan_u8(const uint8_t* q, const uint8_t* db, const uint8_t* digits, size_t n_pad, int n, int nq, int k,
                               int kprime, int m_half, uint32_t pos_base, int n_cta, int s_max, const int* d_pieces,
-                              uint64_t* cand, int* cand_cnt, float* cand_thr, uint32_t* gthr, cudaStream_t stream);
+                              uint64_t* cand, int* cand_cnt, float* cand_thr, uint32_t* gthr, cudaStream_t stream,
+                              uint32_t* range_cut = nullptr);  // range mode (see launch_tc_scan_ts)
+// range mode of launch_tc_scan_u8: gthr[i] = the int bits of query i's accumulator threshold (a row passes when
+// acc > T_acc) for the floored radius radii[i]; q: staged byte queries [q_pad][128]
+cudaError_t launch_tc_range_threshold_u8(const uint8_t* q, int nq, const float* radii, int m_half, uint32_t* gthr,
+                                         cudaStream_t stream);
 // 3xTF32 operand split: dst[r] = [hi | lo | hi] (layout 0, database) or [hi | hi | lo] (layout 1, queries) of
 // scale * src[r], hi = the TF32-exact part, lo = the TF32-exact part of the rest; dst rows are 3 * row_words long
 cudaError_t launch_tc_split_rows(const float* src, size_t rows, int row_words, float scale, int layout, float* dst,

@@ -36,7 +36,8 @@
 // warp-cooperative compaction of the buffer; shared between the CTAs of one query through a per-query word.
 // Batched range queries (DESIGN.md K5b): the TS and pair kernels have a RANGE variant whose thresholds are fixed per
 // query (tc_range_threshold_kernel turns the radius into the pass-1 rank domain, widened by the certificate's error
-// band); survivors are kept in position order up to a position cut, and range_scan.cu verifies them.
+// band); survivors are kept in position order up to a position cut, and range_scan.cu verifies them.  The u8 kernel's
+// RANGE variant does the same on exact integer accumulators (tc_range_threshold_u8_kernel, error bound 1).
 #include <cuda.h>
 
 #include <algorithm>
@@ -1539,6 +1540,7 @@ struct U8Params {
   const uint8_t* q;         // [q_pad][128] query bytes (zero rows past nq)
   int m_half;               // M = ceil(max |x|^2 / 2)
   unsigned long long* counters;
+  uint32_t* cand_cut;       // range mode, instead of cand_thr (see TcParams)
 };
 
 __device__ __forceinline__ void umma_i8_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
@@ -1582,11 +1584,14 @@ __device__ __forceinline__ int u8_acc_of_rank(float rank, int m_half) {  // pass
   return m_half - (__float2int_rd(rank) >> 1) - ((__float2int_rd(rank) & 1) ? 1 : 0) + 0;
 }
 
-// per-lane selection over one 64-column tile (integer twin of epi_select_tile): acc > thr passes
-template <bool REG>
+// per-lane selection over one 64-column tile (integer twin of epi_select_tile): acc > thr passes.
+// RANGE: keys are appended in position order; a full buffer records its first dropped position in *cut and the row
+// stops selecting (thr = INT_MAX: no accumulator passes).
+template <bool REG, bool RANGE = false>
 __device__ __forceinline__ void epi_select_tile_i(const int (&r0)[32], const int (&r1)[32], const int (&g0)[4],
                                                   const int (&g1)[4], uint32_t pos0, uint64_t* buf, int& cnt, int& thr,
-                                                  int (&tk)[TS_RK], uint32_t* gthr, int m_half) {
+                                                  int (&tk)[TS_RK], uint32_t* gthr, int m_half, int cap = 0,
+                                                  uint32_t* cut = nullptr) {
   unsigned gm = 0;
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
@@ -1615,6 +1620,14 @@ __device__ __forceinline__ void epi_select_tile_i(const int (&r0)[32], const int
       const int lo4 = (jj & 2) ? ((jj & 1) ? v[3] : v[2]) : ((jj & 1) ? v[1] : v[0]);
       const int hi4 = (jj & 2) ? ((jj & 1) ? v[7] : v[6]) : ((jj & 1) ? v[5] : v[4]);
       const int x = (jj & 4) ? hi4 : lo4;
+      if constexpr (RANGE) {
+        if (cnt == cap) {
+          *cut = pos0 + 8 * q + jj;
+          thr = 0x7FFFFFFF;
+          gm = 0;
+          break;
+        }
+      }
       if (!REG || x > thr) {
         buf[cnt] = ((uint64_t)__float_as_uint(u8_rank_of(x, m_half)) << 32) | (uint64_t)(pos0 + 8 * q + jj);
         ++cnt;
@@ -1636,7 +1649,10 @@ __device__ __forceinline__ void epi_select_tile_i(const int (&r0)[32], const int
   }
 }
 
-template <int KPL, bool REG>
+// RANGE: batched range queries -- every row's threshold is its query's fixed accumulator threshold T_acc (p.gthr, the
+// int bits written by tc_range_threshold_u8_kernel), no compaction, no refresh; a list whose buffer fills stores the
+// position of its first dropped survivor in p.cand_cut.
+template <int KPL, bool REG, bool RANGE = false>
 __global__ void __launch_bounds__(TS_THREADS, 1)
 tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmN, const U8Params p) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -1776,7 +1792,8 @@ tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
       uint64_t* buf = p.cand + (unit * TC_QB + h * TC_BM + row) * (size_t)p.cap;
       uint32_t* gthr = p.gthr + qrow;
       int cnt = 0;
-      int thr = row_valid ? -1 : 0x7FFFFFFF;  // pass iff acc > thr (accumulators are >= 0)
+      int thr = !row_valid ? 0x7FFFFFFF : RANGE ? (int)*gthr : -1;  // pass iff acc > thr (accumulators are >= 0)
+      uint32_t cut = 0xFFFFFFFFu;
       int tk[TS_RK];
 #pragma unroll
       for (int i = 0; i < TS_RK; ++i) tk[i] = -1;
@@ -1797,7 +1814,8 @@ tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
         tc_fence_before();
         mbar_arrive(afull_bar);
       }
-      const int guard = REG ? p.cap - TS_BN - 1 : p.hwm;
+      // a row above this many keys sends its warp to the slow path (RANGE: a full row has stopped selecting)
+      const int guard = RANGE ? p.cap : REG ? p.cap - TS_BN - 1 : p.hwm;
       for (int tile = t_begin; tile < t_end; ++tile) {
         uint32_t v0[32], v1[32];
         NB_TACC(c_proc, te);
@@ -1833,12 +1851,14 @@ tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
         }
         const int mm = max3i(max(max3i(g0[0], g0[1], g0[2]), max3i(g0[3], g1[0], g1[1])), g1[2], g1[3]);
         const int vtile = p.n - tile * TS_BN;
-        const bool uni = ((((tile - t_begin) & p.refresh_mask) == 0) & !NB200_DBG(p.debug, 4)) | (vtile < TS_BN);
+        // (RANGE: the thresholds are fixed, the only warp-uniform reason is the shard's last, partial tile)
+        const bool uni = RANGE ? vtile < TS_BN
+                               : ((((tile - t_begin) & p.refresh_mask) == 0) & !NB200_DBG(p.debug, 4)) | (vtile < TS_BN);
         const bool mine = (mm > thr) | (cnt > guard);
         if (!uni && !__any_sync(FULL, mine)) continue;
         if (NB200_DBG(p.debug, 2) && tile - t_begin > 64) continue;  // timing experiment: the fast path only
         // ------------------------------------------------------------------ slow path
-        if (((tile - t_begin) & p.refresh_mask) == 0 && row_valid)
+        if (!RANGE && ((tile - t_begin) & p.refresh_mask) == 0 && row_valid)
           thr = max(thr, u8_acc_of_rank(f32_from_ordered(*gthr), p.m_half));
         if (vtile < TS_BN) {  // rows past the end of the shard: never candidates
 #pragma unroll
@@ -1852,7 +1872,7 @@ tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
             g1[q] = group_max8(r1, q);
           }
         }
-        unsigned need = __ballot_sync(FULL, cnt > p.cap - TS_BN - 1);
+        unsigned need = RANGE ? 0u : __ballot_sync(FULL, cnt > p.cap - TS_BN - 1);
         while (need) {
           ++ctr[2];
           const int src = __ffs(need) - 1;
@@ -1864,9 +1884,9 @@ tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
         ++ctr[1];
         const uint32_t pos_tile = p.pos_base + (uint32_t)(tile * TS_BN);
         if (mm > thr || vtile < TS_BN) {
-          epi_select_tile_i<REG>(r0, r1, g0, g1, pos_tile, buf, cnt, thr, tk, gthr, p.m_half);
+          epi_select_tile_i<REG, RANGE>(r0, r1, g0, g1, pos_tile, buf, cnt, thr, tk, gthr, p.m_half, p.cap, &cut);
         }
-        if constexpr (REG) continue;
+        if constexpr (REG || RANGE) continue;
         const unsigned pend = __ballot_sync(FULL, cnt > p.hwm);
         if (pend) {
           ++ctr[3];
@@ -1878,7 +1898,8 @@ tc_scan_u8_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
       }
       const size_t slot = unit * TC_QB + h * TC_BM + row;
       p.cand_cnt[slot] = row_valid ? cnt : 0;
-      p.cand_thr[slot] = thr < 0 ? __int_as_float(0x7F800000) : u8_rank_of(thr, p.m_half);
+      if constexpr (RANGE) p.cand_cut[slot] = cut;
+      else p.cand_thr[slot] = thr < 0 ? __int_as_float(0x7F800000) : u8_rank_of(thr, p.m_half);
     }
     if (p.counters && lane == 0) {
       for (int i = 0; i < 4; ++i) atomicAdd(p.counters + i, (unsigned long long)ctr[i]);
@@ -2277,6 +2298,34 @@ __global__ void tc_range_threshold_kernel(const float* __restrict__ q, int nq, i
   gthr[qi] = f32_ordered(nextafterf(__double2float_ru(t + (double)E), INFINITY));
 }
 
+// uint8 byte rows (tc_scan_u8_kernel): the radius as a threshold in the accumulator domain, one warp per query.
+// acc = q.x + M - ceil(|x|^2 / 2), so 2 (M - acc) = d - |q|^2 + (|x|^2 odd) with d = |q|^2 + |x|^2 - 2 q.x, all exact
+// integers.  For R = floor(radius), d <= R gives 2 (M - acc) <= R - |q|^2 + 1, i.e. acc > T_acc with
+// T_acc = M - floor((R - |q|^2 + 1) / 2) - 1.  Invariant: every row with d <= R passes; the only other rows that pass
+// lie at d = R + 1 with |x|^2 even, and verification drops them.  Stored as the int bits of T_acc, clamped to -1 (every
+// accumulator passes: R >= 2^24 exceeds every distance of 128 bytes, or R = +inf) and INT_MAX (none can: R < 0 or NaN).
+// (u8_acc_of_rank is exact for integral ranks only: the radius in the rank domain is not one.)
+__global__ void tc_range_threshold_u8_kernel(const uint8_t* __restrict__ q, int nq, const float* __restrict__ radii,
+                                             int m_half, uint32_t* __restrict__ gthr) {
+  const int qi = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+  if (qi >= nq) return;
+  const uchar4 v = reinterpret_cast<const uchar4*>(q + (size_t)qi * U8_ROW)[lane];
+  const int qn2 = __reduce_add_sync(FULL, (int)v.x * v.x + (int)v.y * v.y + (int)v.z * v.z + (int)v.w * v.w);
+  if (lane != 0) return;
+  const float r = radii[qi];
+  long long t;
+  if (!(r >= 0.f)) {
+    t = 0x7FFFFFFF;
+  } else if (r >= 16777216.f) {
+    t = -1;
+  } else {
+    const long long b = (long long)r - qn2 + 1;              // (long long)r = floor(r) for r >= 0
+    const long long half = b >= 0 ? b / 2 : -((1 - b) / 2);  // floor(b / 2), also for b < 0
+    t = (long long)m_half - half - 1;
+  }
+  gthr[qi] = (uint32_t)(int)std::max(-1LL, std::min(0x7FFFFFFFLL, t));
+}
+
 // ---------------------------------------------------------------- operand preparation
 // A' = scale * q (scale = -2 for l2, -1 otherwise) into a buffer padded to 256-row blocks; also
 // flags a batch that is not TF32-exact (any of the 13 low mantissa bits set).
@@ -2458,7 +2507,8 @@ cudaError_t launch_u8_norm_digits(const int* norm2, int n, int n_pad, int m_half
 
 cudaError_t launch_tc_scan_u8(const uint8_t* q, const uint8_t* db, const uint8_t* digits, size_t n_pad, int n, int nq, int k,
                               int kprime, int m_half, uint32_t pos_base, int n_cta, int s_max, const int* d_pieces,
-                              uint64_t* cand, int* cand_cnt, float* cand_thr, uint32_t* gthr, cudaStream_t stream) {
+                              uint64_t* cand, int* cand_cnt, float* cand_thr, uint32_t* gthr, cudaStream_t stream,
+                              uint32_t* range_cut) {
   if (n <= 0 || nq <= 0) return cudaSuccess;
   CUtensorMap tmB, tmN;
   if (!make_tmap_u8(&tmB, db, n_pad, U8_ROW, TS_BN) || !make_tmap_u8(&tmN, digits, n_pad, U8_NROW, TS_BN)) return cudaErrorUnknown;
@@ -2482,6 +2532,8 @@ cudaError_t launch_tc_scan_u8(const uint8_t* q, const uint8_t* db, const uint8_t
   p.q = q;
   p.m_half = m_half;
   p.counters = nullptr;
+  p.cand_cut = range_cut;
+  if (range_cut) p.cap = tc_range_cap();
   {
     const char* dbg = nb200_env("NB200_TC_DEBUG");
     p.debug = dbg ? atoi(dbg) : 0;
@@ -2506,18 +2558,20 @@ cudaError_t launch_tc_scan_u8(const uint8_t* q, const uint8_t* db, const uint8_t
   p.n_stage = 16;
   const size_t smem = 1024 + (size_t)p.n_stage * U8_STAGE + (2 * 16 + 4 * U8_NBUF + 2) * 8 + 16;
   cudaError_t e;
-#define NB_U8(KPL, REG)                                                                                          \
-  e = cudaFuncSetAttribute(tc_scan_u8_kernel<KPL, REG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-  if (e != cudaSuccess) return e;                                                                                \
-  tc_scan_u8_kernel<KPL, REG><<<n_cta, TS_THREADS, smem, stream>>>(tmB, tmN, p);
-  if (k + 4 <= TS_RK && kprime <= k + 6 && p.cap == 256) {
+#define NB_U8(KPL, REG, RANGE)                                                                                          \
+  e = cudaFuncSetAttribute(tc_scan_u8_kernel<KPL, REG, RANGE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+  if (e != cudaSuccess) return e;                                                                                       \
+  tc_scan_u8_kernel<KPL, REG, RANGE><<<n_cta, TS_THREADS, smem, stream>>>(tmB, tmN, p);
+  if (range_cut) {
+    NB_U8(8, false, true);
+  } else if (k + 4 <= TS_RK && kprime <= k + 6 && p.cap == 256) {
     p.kprime = TS_RK;
     p.slack = 8;
-    NB_U8(8, true);
+    NB_U8(8, true, false);
   } else if (p.cap == 256) {
-    NB_U8(8, false);
+    NB_U8(8, false, false);
   } else {
-    NB_U8(16, false);
+    NB_U8(16, false, false);
   }
 #undef NB_U8
   e = cudaGetLastError();
@@ -3000,6 +3054,13 @@ cudaError_t launch_tc_range_threshold(const float* q, int nq, int row_words, int
   pass1_eps(row_words, &eps_exact, &eps_inexact);
   tc_range_threshold_kernel<<<(nq + 7) / 8, 256, 0, stream>>>(q, nq, row_words, mode, take_sqrt, radii, x_max,
                                                               eps_inexact, eps_exact, db_inexact, gthr);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_tc_range_threshold_u8(const uint8_t* q, int nq, const float* radii, int m_half, uint32_t* gthr,
+                                         cudaStream_t stream) {
+  if (nq <= 0) return cudaSuccess;
+  tc_range_threshold_u8_kernel<<<(nq + 7) / 8, 256, 0, stream>>>(q, nq, radii, m_half, gthr);
   return cudaGetLastError();
 }
 
