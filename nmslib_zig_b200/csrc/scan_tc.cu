@@ -1515,7 +1515,7 @@ tc_scan_ts_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant
 //     >= 0 written as 32 base-255 "digits" d_j(x) (one more 32-byte k-block per row, against the constant operand
 //     row c = [1, 255, 255, ...]),      acc = q.x + sum_j c_j d_j(x) = q.x + V(x),
 //     so that  2 (M - acc) = |x|^2 - 2 q.x + (|x|^2 odd)  is the pass-1 rank: exact up to +1, larger acc = nearer.
-//     One extra K = 32 MMA per tile and half; needs max |x|^2 <= 4 032 060 (else the engine keeps the widened path);
+//     One extra K = 32 MMA per tile and half; needs max |x|^2 <= 4 032 059 (else the engine keeps the widened path);
 //   * tensor memory: [0, 128) operand rows (per half 32 columns of query bytes + 8 columns of constants),
 //     [128, 512) THREE accumulator buffers x two halves x 64 columns -- one more than the TF32 kernel has room for,
 //     which is what absorbs the epilogue's jitter now that a tile's MMAs take ~320 clk instead of ~1100;
@@ -2454,15 +2454,17 @@ bool make_tmap_u8(CUtensorMap* map, const void* base, size_t rows, int row_bytes
 }
 
 // uint8 rows: int32 |x|^2 per row (aux, from launch_row_aux) -> the 32 norm digits of V(x) = m_half - ceil(|x|^2 / 2)
-// (d0 = V mod 255, then floor(V / 255) spread over 31 digits of at most 255); padding rows get V = 0
+// (rest = floor(V / 255) spread over 31 digits of at most 255, d0 = V - 255 rest); padding rows get V = 0.
+// The 31 digits carry at most 31 * 255 * 255, so rest is capped there and d0 takes the remainder: d0 <= 254 except at
+// V = 255 + 31 * 255 * 255 (a zero row when max |x|^2 is u8_imma_max_norm2(), M = 2 016 030), where d0 = 255
 __global__ void u8_norm_digits_kernel(const int* __restrict__ norm2, int n, int n_pad, int m_half, uint8_t* __restrict__ out) {
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n_pad) return;
   int v = 0;
   if (r < n) v = m_half - ((norm2[r] + 1) >> 1);
   uint32_t w[8];
-  int rest = v / 255;
-  uint32_t d0 = (uint32_t)(v % 255);
+  int rest = min(v / 255, 31 * 255);
+  uint32_t d0 = (uint32_t)(v - 255 * rest);
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
     uint32_t word = 0;
