@@ -284,7 +284,7 @@ typedef struct {
   uint64_t uploaded_rows;    /* rows copied host -> device so far (an append uploads only the new rows) */
   /* nmslib_b200_range_query_batch (b200_devices indexes: counted once per shard) */
   uint64_t range_tc_queries;       /* range queries whose answer came from the tensor-core pass (uint8 included) */
-  uint64_t range_fallback_queries; /* range queries re-run by the per-query exact scan (tensor-core pass uncertified) */
+  uint64_t range_fallback_queries; /* range queries re-run by the per-query exact scan after an uncertified batched pass */
 } nmslib_b200_stats_t;
 nmslib_error_t nmslib_b200_get_stats(nmslib_index_handle_t index, nmslib_b200_stats_t* out);
 
@@ -300,10 +300,11 @@ nmslib_error_t nmslib_b200_get_stats(nmslib_index_handle_t index, nmslib_b200_st
  * nmslib_range_query_fill.  An empty index returns size 0 everywhere.
  * l2, l2sqr, cosinesimil, negdotprod, angulardist and l2sqr_sift run as one tensor-core pass over the rows for the
  * whole batch (a threshold per query, verified with the per-query scan's own distance code; uint8 byte rows on the
- * integer tensor pipe with an exact integer threshold, widened uint8 rows on the TF32 pass); l1, linf, force_exact
- * and, under option tc_pair=0, rows of more than 128 floats use the per-query exact scan, as does
- * any query the tensor-core pass cannot certify (nmslib_b200_stats_t counts both).  A b200_devices index answers
- * over every shard and concatenates the shards' lists in position order. */
+ * integer tensor pipe with an exact integer threshold, widened uint8 rows on the TF32 pass); l1 and linf run as one
+ * pass of the exact CUDA-core scan with a threshold per query, verified the same way.  force_exact and, under option
+ * tc_pair=0, rows of more than 128 floats in the tensor-core spaces use the per-query exact scan, as does any query a
+ * batched pass cannot certify (nmslib_b200_stats_t counts the tensor-core answers and those re-runs).  A
+ * b200_devices index answers over every shard and concatenates the shards' lists in position order. */
 nmslib_error_t nmslib_b200_range_query_batch(nmslib_index_handle_t index, const void* queries,
                                              size_t query_count, size_t elem_count,
                                              const double* radii, nmslib_result_t* results);

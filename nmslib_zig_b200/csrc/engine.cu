@@ -1421,8 +1421,9 @@ Status Engine::range_host(const void* query, size_t elem_count, double radius, s
 // Float spaces with a dot-product form and uint8 run on the tensor cores: radius -> pass-1 threshold T_q (uint8 byte
 // rows: an integer accumulator threshold), the TS / pair / u8 scan in range mode (survivors beating the threshold in
 // position order, a position cut where a list fills), verification of the candidates with the per-query scan's own
-// distance code.  l1 / linf / force_exact, and every query the tensor-core pass cannot certify, take the per-query
-// exact scan (launch_range_scan) inside the same submission.
+// distance code.  l1 / linf run the same way on the CUDA cores: K2 in range mode (scan_exact.cu, T_q from
+// range_threshold), then the same verification.  force_exact, and every query a batched pass cannot certify, take
+// the per-query exact scan (launch_range_scan) inside the same submission.
 // Outputs are staged in CSR form (min(capacity, n) slots per query); a batch whose staging would exceed
 // kRangeStageBytes runs in query chunks.
 namespace {
@@ -1480,6 +1481,8 @@ Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, co
   const bool tc = !force_exact_ && (ts || pair) &&
                   (u8 || u8_widened() || space_ == SPACE_L2 || space_ == SPACE_L2SQR || space_ == SPACE_COSINE ||
                    space_ == SPACE_NEGDOT || space_ == SPACE_ANGULAR);
+  // l1 / linf: K2 in range mode (scan_exact.cu), whatever the row length
+  const bool lp = !force_exact_ && (space_ == SPACE_L1 || space_ == SPACE_LINF);
   Status s = stage_queries_device(queries, false, nq, elem_count, stream_);
   if (!s.ok()) return s;
   // per-query parameters: radii [nq] f32 | caps [nq] i32 | CSR offsets [nq] i64; outputs: counts [nq] | fallback
@@ -1519,8 +1522,56 @@ Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, co
                                         stream_),
                       "range_scan");
   };
+  // the candidate lists of a range-mode scan ([q_pad / 256][s_max][256][list cap]): verification, then the per-query
+  // exact scan of every query it could not certify; *n_fb = how many
+  auto verify = [&](int s_max, size_t* n_fb) {
+    Status v = check_cuda(launch_range_verify(d_db_.as<float>(), d_q_.as<float>(), d_ids_.as<int32_t>(), row_words_, mode,
+                                              take_sqrt, pos_base_, d_radii, d_caps, d_off, d_rcand_.as<uint64_t>(),
+                                              d_rcnt_.as<int>(), d_rcut_.as<uint32_t>(), s_max, tc_range_cap(), 0,
+                                              (int)nq, d_oids, d_odists, d_counts, d_fb_cnt, d_fb_idx, stream_),
+                          "range_verify");
+    if (!v.ok()) return v;
+    ++stats_.kernel_launches;
+    int fb_cnt = 0;
+    v = check_cuda(cudaMemcpyAsync(&fb_cnt, d_fb_cnt, 4, cudaMemcpyDeviceToHost, stream_), "D2H(range fb count)");
+    if (v.ok()) v = check_cuda(cudaStreamSynchronize(stream_), "range batch");
+    if (!v.ok()) return v;
+    *n_fb = (size_t)fb_cnt;
+    if (fb_cnt > 0) {
+      std::vector<int> fb(fb_cnt);
+      v = check_cuda(cudaMemcpyAsync(fb.data(), d_fb_idx, fb.size() * 4, cudaMemcpyDeviceToHost, stream_), "D2H(range fb list)");
+      if (v.ok()) v = check_cuda(cudaStreamSynchronize(stream_), "range batch");
+      for (size_t j = 0; j < fb.size() && v.ok(); ++j) v = exact((size_t)fb[j]);
+    }
+    return v;
+  };
   size_t n_fb = 0;
-  if (!tc) {
+  if (lp) {
+    // K2 split like run_seq_exact (>= 2 CTAs per SM worth of work), into at most 2^15 / cap splits: range_verify_kernel
+    // sorts s_max * cap positions in a power-of-two shared buffer of at most 200 KB
+    const int bq = scan_exact_block_queries(), bn = scan_exact_block_points(), cap = tc_range_cap();
+    const int n_tiles = (int)((n_dev_ + bn - 1) / bn);
+    const int q_blocks = (int)((nq + bq - 1) / bq);
+    const int want = (2 * sm_count_ + q_blocks - 1) / q_blocks;
+    const int n_split = std::max(1, std::min({want, n_tiles, (1 << 15) / cap}));
+    const int tiles_per_split = (n_tiles + n_split - 1) / n_split;
+    const int s_max = (n_tiles + tiles_per_split - 1) / tiles_per_split;
+    const size_t lists = round_up(nq, (size_t)tc_block_queries()) * s_max;  // (every list is written by the scan)
+    if (!(s = check_cuda(d_rcand_.ensure(lists * cap * 8), "cudaMalloc(range cand)")).ok()) return s;
+    if (!(s = check_cuda(d_rcnt_.ensure(lists * 4), "cudaMalloc(range cand_cnt)")).ok()) return s;
+    if (!(s = check_cuda(d_rcut_.ensure(lists * 4), "cudaMalloc(range cut)")).ok()) return s;
+    if (!(s = check_cuda(cudaMemsetAsync(d_fb_cnt, 0, 4, stream_), "memset(range fb count)")).ok()) return s;
+    scan_begin(stream_);
+    s = check_cuda(launch_scan_exact_range(mode, d_db_.p, d_q_.p, (int)n_dev_, (int)nq, row_words_, pos_base_, d_radii,
+                                           cap, d_rcand_.as<uint64_t>(), d_rcnt_.as<int>(), d_rcut_.as<uint32_t>(), s_max,
+                                           tiles_per_split, stream_),
+                   "scan_exact(range)");
+    scan_end(stream_);
+    if (!s.ok()) return s;
+    ++stats_.kernel_launches;
+    if (!(s = verify(s_max, &n_fb)).ok()) return s;
+    stats_.range_fallback_queries += n_fb;
+  } else if (!tc) {
     for (size_t i = 0; i < nq && s.ok(); ++i) s = exact(i);
     if (!s.ok()) return s;
   } else {
@@ -1580,25 +1631,8 @@ Status Engine::range_chunk(const void* queries, size_t nq, size_t elem_count, co
                    u8 ? "tc_scan_u8(range)" : ts ? "tc_scan_ts(range)" : "tc_scan_pair(range)");
     scan_end(stream_);
     if (!s.ok()) return s;
-    s = check_cuda(launch_range_verify(d_db_.as<float>(), d_q_.as<float>(), d_ids_.as<int32_t>(), row_words_, mode,
-                                       take_sqrt, pos_base_, d_radii, d_caps, d_off, d_rcand_.as<uint64_t>(),
-                                       d_rcnt_.as<int>(), d_rcut_.as<uint32_t>(), s_max, (int)cap, 0, (int)nq, d_oids,
-                                       d_odists, d_counts, d_fb_cnt, d_fb_idx, stream_),
-                   "range_verify");
-    if (!s.ok()) return s;
-    stats_.kernel_launches += 3;
-    int fb_cnt = 0;
-    s = check_cuda(cudaMemcpyAsync(&fb_cnt, d_fb_cnt, 4, cudaMemcpyDeviceToHost, stream_), "D2H(range fb count)");
-    if (s.ok()) s = check_cuda(cudaStreamSynchronize(stream_), "range batch");
-    if (!s.ok()) return s;
-    n_fb = (size_t)fb_cnt;
-    if (n_fb > 0) {
-      std::vector<int> fb(n_fb);
-      s = check_cuda(cudaMemcpyAsync(fb.data(), d_fb_idx, n_fb * 4, cudaMemcpyDeviceToHost, stream_), "D2H(range fb list)");
-      if (s.ok()) s = check_cuda(cudaStreamSynchronize(stream_), "range batch");
-      for (size_t j = 0; j < n_fb && s.ok(); ++j) s = exact((size_t)fb[j]);
-      if (!s.ok()) return s;
-    }
+    stats_.kernel_launches += 2;
+    if (!(s = verify(s_max, &n_fb)).ok()) return s;
     stats_.range_tc_queries += nq - n_fb;
     stats_.range_fallback_queries += n_fb;
   }

@@ -146,7 +146,9 @@ struct Stats {
   double last_kernel_ms = 0, last_total_ms = 0, last_scan_ms = 0, scan_ms_sum = 0;
   uint64_t scan_count = 0;
   uint64_t fallback_queries = 0, device_bytes = 0, split_queries = 0, uploaded_rows = 0;
-  uint64_t range_tc_queries = 0, range_fallback_queries = 0;  // batched range queries (range_batch_host)
+  // batched range queries (range_batch_host): answered by the tensor-core pass / re-run by the per-query exact scan
+  // after an uncertified batched pass
+  uint64_t range_tc_queries = 0, range_fallback_queries = 0;
 };
 
 class Engine {

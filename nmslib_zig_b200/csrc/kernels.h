@@ -41,6 +41,12 @@ cudaError_t launch_scan_exact(int mode, const void* db, const void* queries, con
                               uint64_t* partial, int n_split, int tiles_per_split, cudaStream_t stream,
                               const int* d_nq = nullptr,   // d_nq: query count read on the device (<= nq)
                               uint64_t* glists = nullptr);  // k > scan_exact_smem_k(): scratch of scan_exact_glists_bytes()
+// Range mode (batched range queries, mode SCAN_L1 / SCAN_LINF): every query's fixed threshold comes from radii[nq];
+// cand / cand_cnt / cut are the candidate lists range_verify_kernel reads (see launch_range_verify), n_split lists
+// of list_cap keys per query, written for every query row of the grid (queries padded to 256-query blocks).
+cudaError_t launch_scan_exact_range(int mode, const void* db, const void* queries, int n, int nq, int row_words,
+                                    uint32_t pos_base, const float* radii, int list_cap, uint64_t* cand, int* cand_cnt,
+                                    uint32_t* cut, int n_split, int tiles_per_split, cudaStream_t stream);
 int scan_exact_max_k();
 int scan_exact_smem_k();
 size_t scan_exact_glists_bytes(int nq, int k, int n_split);

@@ -18,6 +18,10 @@
 // distance matrix never leaves registers: every value is compared with its query's
 // current k-th best (shared memory); survivors (rare once warm) go through a small
 // shared-memory queue into per-query sorted lists of 64-bit (distance, position) keys.
+//
+// RANGE variant (batched range queries over l1 / linf, DESIGN.md K5b): the same main loop, but every query row has a
+// fixed threshold T_q (range_threshold) for the whole scan, and survivors go straight into the query's candidate
+// list of this split, in the layout range_verify_kernel (range_scan.cu) reads.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -86,13 +90,44 @@ __device__ __forceinline__ float cosine_exact(float dot, float n_x, float n_q) {
 // AngularDistance, distcomp_scalar.cc:254-258
 __device__ __forceinline__ float angular_exact(float dot, float n_x, float n_q) { return acosf(nsp_exact(dot, n_x, n_q)); }
 
+// Batched range queries: the pass-1 threshold T_q of radius r (a row is a candidate when its pass-1 value <= T_q).
+// Invariant: every row whose range_row_dist value is <= r has pass-1 value <= T_q.
+// Both sums use the same terms t_i = |fl(x_i - y_i)| (fabsf of the same subtraction; fl(q - x) = -fl(x - q)); pass 1
+// adds them sequentially over the row, range_row_dist in lane-strided float4 groups and a butterfly.
+//  - linf: the max of one set of terms does not depend on the order, and fmaxf skips NaN terms the same way in
+//    both, so the two values are equal bit for bit: T_q = r.
+//  - l1: the terms are >= 0, so any summation order of the D = row_words terms (padding words add exact zeros) is
+//    within gamma S of the exact sum S, gamma = (D - 1) u / (1 - (D - 1) u), u = 2^-24 (no underflow error: fp32
+//    addition is exact in the subnormal range; no overflow below T_q: every partial sum is <= the final sum).
+//    verified <= r  =>  S <= r / (1 - gamma)  =>  pass1 <= S (1 + gamma) <= r (1 + gamma) / (1 - gamma), evaluated in
+//    double, rounded up to float and raised by one more ulp for the double rounding; an overflow becomes +inf.
+// r = +inf admits every row, +inf values included; a NaN radius admits none (value <= NaN is false, as it is for the
+// per-query scan); NaN values (a NaN term) are NaN in both sums and never selected.
 template <int MODE>
+__device__ __forceinline__ float range_threshold(float r, int row_words) {
+  if constexpr (MODE == SCAN_LINF) {
+    return r;
+  } else {
+    const double x = (row_words - 1) * 0x1p-24, gamma = x / (1.0 - x);
+    if (!(gamma < 1.0)) return INFINITY;  // rows of 2^23 words and more: no bound, verification filters everything
+    return nextafterf(__double2float_ru((double)r * (1.0 + gamma) / (1.0 - gamma)), INFINITY);
+  }
+}
+
+// RANGE (MODE SCAN_L1 / SCAN_LINF only): partial / d_nq / glists unused; k = list capacity; radii[nq] the float radii;
+// cand [q_blocks of 256][n_split][256][k] keys (ordered pass-1 value << 32 | position), in arrival order;
+// cand_cnt / cut [q_blocks of 256][n_split][256], written for every query row of the CTA (a 128-query CTA fills one
+// half of a 256-query block; the split index is the list index).  A full list stores the smallest position it
+// dropped in its cut and stops selecting in the next tile, so every survivor below the cut was kept.
+template <int MODE, bool RANGE = false>
 __global__ void __launch_bounds__(NT, (MODE == SCAN_SIFT) ? 1 : 1)
 scan_exact_kernel(const uint32_t* __restrict__ db, const uint32_t* __restrict__ qs,
                   const void* __restrict__ db_aux_v, const void* __restrict__ q_aux_v, int n, int nq,
                   int row_words, int k, int tiles_per_split, uint32_t pos_base,
                   uint64_t* __restrict__ partial, int n_split, const int* __restrict__ d_nq,
-                  uint64_t* __restrict__ glists) {
+                  uint64_t* __restrict__ glists, const float* __restrict__ radii, uint64_t* __restrict__ cand,
+                  int* __restrict__ cand_cnt, uint32_t* __restrict__ cut) {
+  static_assert(!RANGE || MODE == SCAN_L1 || MODE == SCAN_LINF, "range mode: l1 / linf");
   using acc_t = typename Acc<MODE>::type;
   if (d_nq) {  // query count decided on the device (the re-run of uncertified queries): surplus blocks leave at once
     nq = min(nq, *d_nq);
@@ -104,11 +139,12 @@ scan_exact_kernel(const uint32_t* __restrict__ db, const uint32_t* __restrict__ 
   // has no capacity limit (knnqueue.h:55-64) -- this block's slice of a global scratch array (slower, but unbounded)
   uint64_t* slists = reinterpret_cast<uint64_t*>(tiles + NSTAGE * (BQ + BN) * LDW);
   uint64_t* lists = glists ? glists + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * (size_t)BQ * k : slists;
-  uint64_t* thr_key = slists + (glists ? 0 : (size_t)BQ * k);                   // BQ
+  uint64_t* thr_key = slists + (glists || RANGE ? 0 : (size_t)BQ * k);         // BQ (RANGE: no lists; k = list cap)
   uint64_t* qkey = thr_key + BQ;                                                // QCAP
   uint32_t* thr_fast = reinterpret_cast<uint32_t*>(qkey + QCAP);                // BQ (bit pattern)
   int* cnt = reinterpret_cast<int*>(thr_fast + BQ);                             // BQ
   uint16_t* qrow = reinterpret_cast<uint16_t*>(cnt + BQ);                       // QCAP
+  uint32_t* rcut = reinterpret_cast<uint32_t*>(thr_key);  // RANGE: BQ cuts (thr_key unused); thr_fast = T_q
   __shared__ int qcount;
 
   const int tid = threadIdx.x;
@@ -121,7 +157,13 @@ scan_exact_kernel(const uint32_t* __restrict__ db, const uint32_t* __restrict__ 
   const int n_tiles = max(t1 - t0, 0);
   const int n_kb = row_words / BW;
 
-  if (tid < BQ) {
+  if constexpr (RANGE) {
+    if (tid < BQ) {  // (padding rows: -inf selects nothing)
+      thr_fast[tid] = q0 + tid < nq ? __float_as_uint(range_threshold<MODE>(radii[q0 + tid], row_words)) : 0xFF800000u;
+      rcut[tid] = 0xFFFFFFFFu;
+      cnt[tid] = 0;
+    }
+  } else if (tid < BQ) {
     thr_key[tid] = KEY_MAX;
     cnt[tid] = 0;
     if constexpr (MODE == SCAN_SIFT) thr_fast[tid] = 0x7FFFFFFFu;
@@ -223,7 +265,9 @@ scan_exact_kernel(const uint32_t* __restrict__ db, const uint32_t* __restrict__ 
     uint64_t pend = 0;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      const uint32_t tbits = thr_fast[ty + 16 * i];
+      uint32_t tbits = thr_fast[ty + 16 * i];
+      if constexpr (RANGE)  // a list that dropped a survivor in an earlier tile has stopped selecting
+        if (rcut[ty + 16 * i] < pos_base + (uint32_t)(tile * BN)) tbits = 0xFF800000u;
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         bool pass;
@@ -242,8 +286,31 @@ scan_exact_kernel(const uint32_t* __restrict__ db, const uint32_t* __restrict__ 
       }
     }
 
+    // ---------------- RANGE: survivors straight into the query's list of this split ----------------
+    // (arrival order: verification sorts by position.)  The stop test above compares the cut with this tile's first
+    // position, so a drop in this tile, whether other threads see it yet or not, never stops this tile's selection:
+    // every survivor is either kept or folded into the cut, and the cut is the smallest dropped position.
+    if constexpr (RANGE) {
+      if (pend) {
+        const size_t list0 = ((size_t)(blockIdx.y >> 1) * n_split + split) * (2 * BQ) + (blockIdx.y & 1) * BQ;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            if (pend & (1ull << (i * 8 + j))) {
+              const int row = ty + 16 * i;
+              const uint32_t pos = pos_base + (uint32_t)(tile * BN + tx + 16 * j);
+              const int e = atomicAdd(&cnt[row], 1);
+              if (e < k) cand[(list0 + row) * k + e] = make_key(f32_ordered(acc[i][j]), pos);
+              else atomicMin(&rcut[row], pos);
+            }
+          }
+        }
+      }
+    }
+
     // ---------------- slow path: queue the survivors, drain into sorted lists ----------------
-    while (true) {
+    while (!RANGE) {
       if (!__syncthreads_or(pend != 0ull)) break;
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
@@ -318,6 +385,15 @@ scan_exact_kernel(const uint32_t* __restrict__ db, const uint32_t* __restrict__ 
   cp_async_wait<0>();
   __syncthreads();
 
+  if constexpr (RANGE) {
+    if (tid < BQ) {
+      const size_t slot = ((size_t)(blockIdx.y >> 1) * n_split + split) * (2 * BQ) + (blockIdx.y & 1) * BQ + tid;
+      cand_cnt[slot] = min(cnt[tid], k);
+      cut[slot] = rcut[tid];
+    }
+    return;
+  }
+
   // ---------------- write this split's sorted partial list ----------------
   if (tid < BQ) {
     const int q = q0 + tid;
@@ -360,7 +436,8 @@ cudaError_t launch_scan_exact(int mode, const void* db, const void* queries, con
   e = cudaFuncSetAttribute(scan_exact_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
   if (e != cudaSuccess) return e;                                                                      \
   scan_exact_kernel<M><<<grid, NT, smem, stream>>>(d, q, db_aux, q_aux, n, nq, row_words, k,           \
-                                                   tiles_per_split, pos_base, partial, n_split, d_nq, glists);
+                                                   tiles_per_split, pos_base, partial, n_split, d_nq, glists, \
+                                                   nullptr, nullptr, nullptr, nullptr);
   switch (mode) {
     case SCAN_L2: NB_LAUNCH(SCAN_L2); break;
     case SCAN_NEGDOT: NB_LAUNCH(SCAN_NEGDOT); break;
@@ -369,6 +446,30 @@ cudaError_t launch_scan_exact(int mode, const void* db, const void* queries, con
     case SCAN_L1: NB_LAUNCH(SCAN_L1); break;
     case SCAN_LINF: NB_LAUNCH(SCAN_LINF); break;
     case SCAN_ANGULAR: NB_LAUNCH(SCAN_ANGULAR); break;
+    default: return cudaErrorInvalidValue;
+  }
+#undef NB_LAUNCH
+  return cudaGetLastError();
+}
+
+cudaError_t launch_scan_exact_range(int mode, const void* db, const void* queries, int n, int nq, int row_words,
+                                    uint32_t pos_base, const float* radii, int list_cap, uint64_t* cand, int* cand_cnt,
+                                    uint32_t* cut, int n_split, int tiles_per_split, cudaStream_t stream) {
+  if (nq <= 0 || n <= 0) return cudaSuccess;
+  const size_t smem = scan_exact_smem(0);
+  dim3 grid(n_split, (nq + BQ - 1) / BQ);
+  const uint32_t* d = static_cast<const uint32_t*>(db);
+  const uint32_t* q = static_cast<const uint32_t*>(queries);
+  cudaError_t e;
+#define NB_LAUNCH(M)                                                                                                  \
+  e = cudaFuncSetAttribute(scan_exact_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);        \
+  if (e != cudaSuccess) return e;                                                                                     \
+  scan_exact_kernel<M, true><<<grid, NT, smem, stream>>>(d, q, nullptr, nullptr, n, nq, row_words, list_cap,          \
+                                                         tiles_per_split, pos_base, nullptr, n_split, nullptr, nullptr, \
+                                                         radii, cand, cand_cnt, cut);
+  switch (mode) {
+    case SCAN_L1: NB_LAUNCH(SCAN_L1); break;
+    case SCAN_LINF: NB_LAUNCH(SCAN_LINF); break;
     default: return cudaErrorInvalidValue;
   }
 #undef NB_LAUNCH
