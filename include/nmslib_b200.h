@@ -210,7 +210,11 @@ nmslib_error_t nmslib_borrow_data_dense(nmslib_index_handle_t index, size_t posi
 
 /* -- persistence (ref :1369-1479).  hnsw indexes are written / read in the
  * reference's optimized-index stream (hnsw.cc:774-806) plus the "<path>.dat"
- * dataset (space.cc:90-105), so files are interchangeable with the reference. */
+ * dataset (space.cc:90-105), so files are interchangeable with the reference.
+ * l2sqr_sift + hnsw (the reference's Hnsw<int>) writes the regular index file
+ * instead (SaveRegularIndexBin, hnsw.cc:810-842: links only); loaded with
+ * DENSE_UINT8_VECTOR it becomes an l2sqr_sift hnsw index over "<path>.dat",
+ * so load_data must be 1 (DATA_IO_FAILED otherwise). */
 nmslib_error_t nmslib_save_index(nmslib_index_handle_t index, const char* path, int save_data);
 nmslib_error_t nmslib_load_index(const char* path, nmslib_data_type_t data_type,
                                  nmslib_dist_type_t dist_type,
@@ -240,8 +244,8 @@ nmslib_error_t nmslib_b200_import_hnsw(nmslib_index_handle_t index, const char* 
 /* Force the lazy device upload now (idempotent). */
 nmslib_error_t nmslib_b200_prepare(nmslib_index_handle_t index);
 
-/* Device-resident batch query: d_queries is [q][elem_count] in device memory,
- * the outputs are device arrays.  d_keys ([q][k] uint64 = ordered(distance) << 32
+/* Device-resident batch query: d_queries is [q][elem_count] in device memory
+ * (float32, or bytes for uint8 indexes, seq_search and hnsw alike), the outputs are device arrays.  d_keys ([q][k] uint64 = ordered(distance) << 32
  * | position) may be NULL.  Runs on `stream` (a cudaStream_t, may be NULL) and does
  * not synchronise.  Missing results (k > n) are id -1 / distance +inf. */
 nmslib_error_t nmslib_b200_knn_device(nmslib_index_handle_t index, const void* d_queries,

@@ -678,7 +678,9 @@ nmslib_error_t nmslib_save_index(nmslib_index_handle_t index, const char* path, 
             Status ps = e->ensure_graph();
             if (!ps.ok()) return NB_STATUS(ps);
           }
-          Status s = nb200::write_hnsw_file(path, e->graph(), e->hnsw_rows_for_save(), e->graph().ext_ids.data());
+          // l2sqr_sift is Hnsw<int> in the reference: it saves the regular index (SaveRegularIndexBin), links only
+          Status s = e->is_u8() ? nb200::write_regular(path, e->graph())
+                                : nb200::write_hnsw_file(path, e->graph(), e->hnsw_rows_for_save(), e->graph().ext_ids.data());
           if (!s.ok()) return NB_STATUS(s);
         } else {
           // SeqSearch has no SaveIndex in the reference (index.h:56-58 throws); we leave a marker
@@ -691,6 +693,34 @@ nmslib_error_t nmslib_save_index(nmslib_index_handle_t index, const char* path, 
         return NB_OK("Index saved successfully");
       },
       NMSLIB_ERROR_DATA_IO_FAILED, "Failed to save index");
+}
+
+// Space::ReadObjectVectorFromBinData (space.cc:60-88): the rows of `path`.dat appended to h; nullptr, or what failed
+static const char* read_dat(const char* path, nmslib_index_handle_t h) {
+  FILE* d = fopen((std::string(path) + ".dat").c_str(), "rb");
+  if (!d) return "Failed to load index: cannot open .dat";
+  uint64_t qty = 0;
+  bool ok = fread(&qty, 8, 1, d) == 1;
+  std::vector<char> buf;
+  for (uint64_t i = 0; ok && i < qty; ++i) {
+    uint64_t buflen = 0;
+    ok = fread(&buflen, 8, 1, d) == 1 && buflen >= 16 && buflen < (1ull << 32);
+    if (!ok) break;
+    buf.resize(buflen);
+    ok = fread(buf.data(), 1, buflen, d) == buflen;
+    if (!ok) break;
+    int32_t id;
+    memcpy(&id, buf.data(), 4);
+    const size_t payload = buflen - 16;
+    uint64_t datalen = 0;  // Object header: id, label, datalength (object.h); must describe this record
+    memcpy(&datalen, buf.data() + 8, 8);
+    ok = datalen == payload && (h->engine->is_u8() ? payload > 4 : (payload >= 4 && payload % 4 == 0));
+    if (!ok) break;
+    const size_t elems = h->engine->is_u8() ? payload - 4 : payload / 4;
+    ok = h->engine->add_rows(buf.data() + 16, 1, elems, &id).ok();
+  }
+  fclose(d);
+  return ok ? nullptr : "Failed to load index: corrupt .dat";
 }
 
 nmslib_error_t nmslib_load_index(const char* path, nmslib_data_type_t data_type, nmslib_dist_type_t dist_type,
@@ -709,37 +739,9 @@ nmslib_error_t nmslib_load_index(const char* path, nmslib_data_type_t data_type,
           nmslib_index_handle_t h = nullptr;
           nmslib_error_t rc = new_index(space, "seq_search", data_type, dist_type, allocator, &h);
           if (rc != NMSLIB_SUCCESS) return rc;
-          if (load_data) {  // Space::ReadObjectVectorFromBinData, space.cc:60-88
-            FILE* d = fopen((std::string(path) + ".dat").c_str(), "rb");
-            if (!d) {
-              nmslib_index_destroy(h);
-              return NB_ERR(NMSLIB_ERROR_DATA_IO_FAILED, "Failed to load index: cannot open .dat");
-            }
-            uint64_t qty = 0;
-            bool ok = fread(&qty, 8, 1, d) == 1;
-            std::vector<char> buf;
-            for (uint64_t i = 0; ok && i < qty; ++i) {
-              uint64_t buflen = 0;
-              ok = fread(&buflen, 8, 1, d) == 1 && buflen >= 16 && buflen < (1ull << 32);
-              if (!ok) break;
-              buf.resize(buflen);
-              ok = fread(buf.data(), 1, buflen, d) == buflen;
-              if (!ok) break;
-              int32_t id;
-              memcpy(&id, buf.data(), 4);
-              const size_t payload = buflen - 16;
-              uint64_t datalen = 0;  // Object header: id, label, datalength (object.h); must describe this record
-              memcpy(&datalen, buf.data() + 8, 8);
-              ok = datalen == payload && (h->engine->is_u8() ? payload > 4 : (payload >= 4 && payload % 4 == 0));
-              if (!ok) break;
-              const size_t elems = h->engine->is_u8() ? payload - 4 : payload / 4;
-              ok = h->engine->add_rows(buf.data() + 16, 1, elems, &id).ok();
-            }
-            fclose(d);
-            if (!ok) {
-              nmslib_index_destroy(h);
-              return NB_ERR(NMSLIB_ERROR_DATA_IO_FAILED, "Failed to load index: corrupt .dat");
-            }
+          if (const char* err = load_data ? read_dat(path, h) : nullptr) {
+            nmslib_index_destroy(h);
+            return NB_ERR(NMSLIB_ERROR_DATA_IO_FAILED, err);
           }
           h->engine->mark_built({});
           *out_handle = h;
@@ -747,13 +749,24 @@ nmslib_error_t nmslib_load_index(const char* path, nmslib_data_type_t data_type,
         }
         // otherwise: the reference's optimized HNSW stream.  The reference hard-codes "hnsw" + "l2"
         // here (nmslib_c.cpp:1421-1429); we read the distance type from the header (SURVEY Q11).
+        // A regular index (flag 0, what l2sqr_sift + hnsw saves) loaded as uint8 is l2sqr_sift over its .dat: the
+        // file holds links only (LoadRegularIndexBin CHECKs that the data set has as many points, hnsw.cc:956-959).
+        uint32_t flag = 1;
+        memcpy(&flag, head, got >= 4 ? 4 : 0);
+        const bool regular_u8 = got >= 4 && flag == 0 && data_type == NMSLIB_DATATYPE_DENSE_UINT8_VECTOR;
+        if (regular_u8 && !load_data)
+          return NB_ERR(NMSLIB_ERROR_DATA_IO_FAILED, "Failed to load index: a regular HNSW index needs its data (load_data=1)");
         nb200::HnswGraph g;
         Status s = nb200::read_hnsw_file(path, &g);
         if (!s.ok()) return NB_STATUS(s);
-        const char* space = g.dist_func == 3 ? "cosinesimil" : g.dist_func == 4 ? "negdotprod" : "l2";
+        const char* space = regular_u8 ? "l2sqr_sift" : g.dist_func == 3 ? "cosinesimil" : g.dist_func == 4 ? "negdotprod" : "l2";
         nmslib_index_handle_t h = nullptr;
         nmslib_error_t rc = new_index(space, "hnsw", data_type, dist_type, allocator, &h);
         if (rc != NMSLIB_SUCCESS) return rc;
+        if (const char* err = regular_u8 ? read_dat(path, h) : nullptr) {
+          nmslib_index_destroy(h);
+          return NB_ERR(NMSLIB_ERROR_DATA_IO_FAILED, err);
+        }
         s = h->engine->adopt_graph(std::move(g));
         if (!s.ok()) {
           nmslib_index_destroy(h);

@@ -440,14 +440,14 @@ Status Engine::adopt_graph(HnswGraph&& g) {
   return Status::OK();
 }
 
-Status Engine::adopt_replica(const HnswGraph& g, const float* search_rows, const int32_t* ids, int dim) {
+Status Engine::adopt_replica(const HnswGraph& g, const void* search_rows, const int32_t* ids, int dim) {
   if (method_ != METHOD_HNSW) return Status::Err(kErrIncompat, "graph replica needs method hnsw");
   if (g.empty() || !search_rows || !ids) return Status::Err(kErrInvalid, "empty graph replica");
   graph_ = g;
   graph_.vectors.clear();
   dim_ = dim;
   n_ = g.total;
-  borrowed_rows_ = search_rows;   // float rows whatever the index's element type (see hnsw_host_rows)
+  borrowed_rows_ = search_rows;
   borrowed_ids_ = ids;
   replica_rows_ = true;
   rows_normalized_ = true;
@@ -502,8 +502,9 @@ Stats Engine::stats() {
   return stats_;
 }
 
-// Rows as the HNSW kernels want them: float32, unit-normalised for cosine (the reference normalises its
-// flat index once at build time, hnsw.cc:441-446), uint8 widened to float (distances stay exact integers).
+// Float rows as the HNSW builders and the float kernels want them: unit-normalised for cosine (the reference normalises
+// its flat index once at build time, hnsw.cc:441-446); uint8 widened to float for the host build only (the search
+// reads the byte rows).
 const float* Engine::hnsw_host_rows() {
   if (replica_rows_) return static_cast<const float*>(borrowed_rows_);  // search-ready rows of the engine replicated
   if (!is_u8_ && (space_ != SPACE_COSINE || rows_normalized_)) return base_f32();
@@ -526,7 +527,7 @@ const float* Engine::hnsw_host_rows() {
 }
 
 int Engine::finalize_kind() const {
-  if (method_ == METHOD_HNSW) return FIN_FLOAT;  // squared / cosine / negdot / (uint8: exact integers held in fp32)
+  if (method_ == METHOD_HNSW) return FIN_FLOAT;  // squared / cosine / negdot / (uint8: exact integers as fp32)
   if (is_u8_) return FIN_INT;  // every uint8 path ends in i32_ordered(int distance) keys (re-rank, dp4a scan)
   // l2 + seq_search reports the root; l2 + hnsw reports the squared distance (SURVEY 0.4)
   if (space_ == SPACE_L2 && method_ == METHOD_SEQ) return FIN_SQRT;
@@ -590,7 +591,7 @@ Status Engine::upload_data() {
   if (!s.ok()) return s;
   const size_t src_row = dev_u8 ? (size_t)dim_ : (size_t)dim_ * 4;
   const void* src = dev_u8 ? (const void*)base_u8() : (const void*)base_f32();
-  if (method_ == METHOD_HNSW) src = hnsw_host_rows();  // float rows; cosine: unit-normalised (hnsw.cc:441-446)
+  if (method_ == METHOD_HNSW && !is_u8_) src = hnsw_host_rows();  // cosine: unit-normalised (hnsw.cc:441-446)
   if (rows_borrowed_) {
     // (adopt_device_rows: the padded rows are already in HBM; ids = positions)
   } else if (u8_widened()) {  // bytes up in 1 M-row chunks, widened to fp32 rows on the device
@@ -761,6 +762,7 @@ Status Engine::ensure_graph_host() {
   const int dist_func = space_ == SPACE_COSINE ? 3 : space_ == SPACE_NEGDOT ? 4 : (dim_ % 16 == 0 ? 1 : 2);
   HnswGraph g;
   Status bs = build_hnsw_host(hnsw_host_rows(), n_, dim_, dist_func, h_ids_.data(), index_params_, &g);
+  if (is_u8_) std::vector<float>().swap(h_hnsw_rows_);  // (widened for the build only: the search reads the bytes)
   if (!bs.ok()) return bs;
   graph_ = std::move(g);
   graph_dirty_ = true;
@@ -774,8 +776,23 @@ Status Engine::build_graph_device() {
   if (!parse_hnsw_build_params(index_params_, &bp, &err)) return Status::Err(kErrBuild, err);
   const int dist_func = space_ == SPACE_COSINE ? 3 : space_ == SPACE_NEGDOT ? 4 : (dim_ % 16 == 0 ? 1 : 2);
   HnswGraph g;
-  Status bs = build_hnsw_device(d_db_.as<float>(), n_, dim_, row_words_, dist_func, h_ids_.data(), bp, device_, &g,
-                                &build_info_);
+  Status bs;
+  if (is_u8_) {
+    // the build scans float rows (TF32 over values 0..255 is exact): widen the byte rows into a temporary buffer
+    const int f_words = (int)round_up((size_t)dim_, tc_kblock_words());
+    const size_t bytes = round_up(n_, scan_exact_block_points()) * f_words * 4;
+    DevBuf wide;
+    bs = check_cuda(wide.ensure(bytes), "cudaMalloc(widened rows)");
+    if (bs.ok()) bs = check_cuda(cudaMemsetAsync(wide.p, 0, bytes, stream_), "memset(widened rows)");
+    if (bs.ok()) bs = check_cuda(launch_widen_u8(d_db_.as<uint8_t>(), n_, dim_, f_words, wide.as<float>(), stream_), "widen_u8");
+    if (bs.ok()) bs = check_cuda(cudaStreamSynchronize(stream_), "widen sync");
+    if (bs.ok())
+      bs = build_hnsw_device(wide.as<float>(), n_, dim_, f_words, dist_func, h_ids_.data(), bp, device_, &g, &build_info_);
+    wide.release();
+  } else {
+    bs = build_hnsw_device(d_db_.as<float>(), n_, dim_, row_words_, dist_func, h_ids_.data(), bp, device_, &g,
+                           &build_info_);
+  }
   if (!bs.ok()) return bs;
   graph_ = std::move(g);
   graph_dirty_ = true;
@@ -896,7 +913,7 @@ Status Engine::run(const void* dq, size_t nq, size_t k, int32_t* d_ids, float* d
   Status s;
   if (method_ == METHOD_HNSW) {
     HnswDeviceGraph g;
-    g.vectors = d_db_.as<float>();
+    g.vectors = d_db_.p;
     g.links0 = d_links0_.as<int32_t>();
     g.links0_cnt = d_links0_cnt_.as<int32_t>();
     g.upper = d_upper_.as<int32_t>();
@@ -909,12 +926,12 @@ Status Engine::run(const void* dq, size_t nq, size_t k, int32_t* d_ids, float* d
     g.maxM0 = graph_.maxM0;
     g.maxlevel = graph_.maxlevel;
     g.enterpoint = (int)graph_.enterpoint;
-    g.dist_kind = graph_.dist_func == 3 ? 1 : graph_.dist_func == 4 ? 2 : 0;
+    g.dist_kind = is_u8_ ? 3 : graph_.dist_func == 3 ? 1 : graph_.dist_func == 4 ? 2 : 0;
     s = check_cuda(d_keys_.ensure(nq * k * 8), "cudaMalloc(keys)");
     if (!s.ok()) return s;
     uint64_t* keys = d_keys ? d_keys : d_keys_.as<uint64_t>();
     scan_begin(stream);
-    s = check_cuda(launch_hnsw_search(g, static_cast<const float*>(dq), (int)nq, (int)k, (int)ef_,
+    s = check_cuda(launch_hnsw_search(g, dq, (int)nq, (int)k, (int)ef_,
                                       d_visited_.as<uint8_t>(), d_epoch_.as<int>(), hnsw_slots_, keys,
                                       d_counters_.as<unsigned long long>(), stream),
                    "hnsw_search");
@@ -1347,8 +1364,6 @@ Status Engine::knn_device(const void* d_queries, size_t nq, size_t elem_count, s
   if (method_ == METHOD_SEQ && !approx_tc && k > (size_t)scan_exact_max_k())
     return Status::Err(kErrTooLarge, "k above " + std::to_string(scan_exact_max_k()) + " is not supported");
   if (method_ == METHOD_HNSW && k > (size_t)hnsw_max_ef()) return Status::Err(kErrTooLarge, "k too large for hnsw");
-  if (is_u8_ && method_ == METHOD_HNSW)
-    return Status::Err(kErrIncompat, "device-resident uint8 queries are not supported for hnsw (use the host entry)");
   cudaStream_t st = stream ? stream : stream_;
   s = stage_queries_device(d_queries, true, nq, elem_count, st, src_pitch);
   if (!s.ok()) return s;
@@ -1714,12 +1729,6 @@ Status Engine::knn_host(const void* queries, size_t nq, size_t elem_count, size_
   if (!(s = check_cuda(h_out_counts_.ensure(nq * 4), "cudaMallocHost(counts)")).ok()) return s;
 
   cudaEventRecord(ev_[0], stream_);
-  if (is_u8_ && method_ == METHOD_HNSW) {  // uint8 + hnsw runs on float rows: widen the queries
-    h_q_widen_.resize(nq * elem_count);
-    const uint8_t* qs = static_cast<const uint8_t*>(queries);
-    for (size_t i = 0; i < nq * elem_count; ++i) h_q_widen_[i] = (float)qs[i];
-    queries = h_q_widen_.data();
-  }
   // chunks of >= 16 K queries only: the search kernel wants a few queries per resident warp (3 552 of them),
   // four chunks of a 10 K batch ran 17.8 ms against 11.5 ms in one launch (profiles/README.md)
   const int n_chunks = (int)std::min<size_t>(kCopyChunks, nq / 16384);
@@ -1727,7 +1736,7 @@ Status Engine::knn_host(const void* queries, size_t nq, size_t elem_count, size_
     // Graph search treats queries independently and its input is large (100 K x 960 floats = 384 MB): copy the
     // batch in chunks on a second stream and search chunk i while chunk i + 1 is still on the bus.
     const size_t bq = std::max(scan_exact_block_queries(), tc_block_queries());
-    const size_t row_bytes = (size_t)row_words_ * 4, src_row = elem_count * 4;
+    const size_t row_bytes = (size_t)row_words_ * 4, src_row = dev_u8_rows() ? elem_count : elem_count * 4;
     const size_t old_cap = d_q_.cap;
     if (!(s = check_cuda(d_q_.ensure(round_up(nq, bq) * row_bytes), "cudaMalloc(queries)")).ok()) return s;
     if (d_q_.cap != old_cap || d_q_dim_ != dim_) {

@@ -88,7 +88,9 @@ class HostSlab {
 struct HnswGraph {
   uint32_t total = 0;
   int dim = 0;
-  int maxM = 0, maxM0 = 0, maxlevel = 0;
+  int maxM = 0, maxM0 = 0, maxlevel = 0;  // maxlevel: the level the greedy descent starts at
+  int M = 0;                              // index-time M (builders, regular files; the optimized stream has none)
+  int file_maxlevel = -1;                 // a regular file's maxlevel_ where it exceeds the entry node's level
   uint32_t enterpoint = 0;
   int dist_func = 0;  // 1 L2Sqr16Ext, 2 L2SqrExt, 3 NormCosine, 4 NegativeDotProduct
   std::vector<float> vectors;      // [total][dim] (cosine: unit norm)
@@ -97,9 +99,13 @@ struct HnswGraph {
   std::vector<int32_t> links0_cnt; // [total]
   std::vector<int32_t> upper;      // concatenated raw upper-level lists
   std::vector<int64_t> upper_off;  // [total], -1 = level 0 only
+  std::vector<int32_t> levels;     // [total] top level of every node
   bool empty() const { return total == 0; }
 };
 Status read_hnsw_file(const std::string& path, HnswGraph* out);
+// The reference's regular index file (Hnsw::SaveRegularIndexBin, hnsw.cc:810-842), what Hnsw<int> (l2sqr_sift) saves:
+// links only, read back by read_hnsw_file.  Needs M and levels.
+Status write_regular(const std::string& path, const HnswGraph& g);
 // vectors / ext_ids: [total][dim] and [total] (the Engine keeps them outside the graph)
 // host-side graph construction (hnsw_build.cpp): rows are float32 (cosine: unit-normalised)
 Status build_hnsw_host(const float* rows, size_t n, int dim, int dist_func, const int32_t* ext_ids,
@@ -180,12 +186,12 @@ class Engine {
   Status set_query_params(const std::vector<std::string>& params);  // hnsw.cc:474-507
   Status import_graph(const std::string& path);
   Status adopt_graph(HnswGraph&& g);
-  // replica of another engine's hnsw index (ShardGroup): a copy of the links over BORROWED search-ready float rows
-  // (cosine: already unit-normalised; uint8: already widened) and ids
-  Status adopt_replica(const HnswGraph& g, const float* search_rows, const int32_t* ids, int dim);
+  // replica of another engine's hnsw index (ShardGroup): a copy of the links over BORROWED search-ready rows
+  // (float: hnsw_rows_for_save(), cosine already unit-normalised; uint8: the host store's byte rows) and ids
+  Status adopt_replica(const HnswGraph& g, const void* search_rows, const int32_t* ids, int dim);
   void release_device();  // frees every device buffer; the next prepare() uploads again
   const HnswGraph& graph() const { return graph_; }
-  const float* hnsw_rows_for_save() { return hnsw_host_rows(); }
+  const float* hnsw_rows_for_save() { return hnsw_host_rows(); }  // float spaces (uint8 graphs save no rows)
   void set_pos_base(uint32_t b) { pos_base_ = b; }
   Status prepare();  // lazy upload; idempotent
   Status ensure_graph_host();  // hnsw: build the graph on the host if none was imported (no GPU needed)
@@ -239,7 +245,8 @@ class Engine {
   // for bit).  NB200_FORCE_EXACT=1 keeps the byte rows and the dp4a scan (K2) instead.
   // Default since round 2: BYTE rows on the integer tensor pipe (tcgen05.mma.kind::i8, tc_scan_u8_kernel) when the
   // rows' norms fit its digit block; the widened TF32 path remains for data beyond that and as option u8_imma=0.
-  bool dev_u8_rows() const { return is_u8_ && method_ == METHOD_SEQ && (force_exact_ || u8_imma_); }
+  // uint8 + hnsw always keeps byte rows: the beam search evaluates them with dp4a (hnsw_search.cu, dist_kind 3).
+  bool dev_u8_rows() const { return is_u8_ && (method_ == METHOD_HNSW || force_exact_ || u8_imma_); }
   bool u8_widened() const { return is_u8_ && method_ == METHOD_SEQ && !force_exact_ && !u8_imma_; }
   bool u8_imma() const { return u8_imma_; }
 
@@ -291,11 +298,11 @@ class Engine {
   std::vector<int32_t> h_ids_;
   const void* borrowed_rows_ = nullptr;    // set by borrow_host_rows: the rows / ids live in another engine's host store
   const int32_t* borrowed_ids_ = nullptr;
-  bool replica_rows_ = false;              // adopt_replica: borrowed_rows_ are search-ready FLOAT rows of an hnsw replica
+  bool replica_rows_ = false;              // adopt_replica: borrowed_rows_ are the search-ready rows of an hnsw replica
   const float* base_f32() const { return borrowed_rows_ ? static_cast<const float*>(borrowed_rows_) : h_f32_.data(); }
   const uint8_t* base_u8() const { return borrowed_rows_ ? static_cast<const uint8_t*>(borrowed_rows_) : h_u8_.data(); }
   const int32_t* base_ids() const { return borrowed_ids_ ? borrowed_ids_ : h_ids_.data(); }
-  std::vector<float> h_hnsw_rows_, h_q_widen_;  // float / normalised rows for hnsw; widened uint8 queries
+  std::vector<float> h_hnsw_rows_;  // float rows for hnsw: cosine normalised; uint8 widened while the host builds
   bool rows_normalized_ = false;
   HnswGraph graph_;
 

@@ -297,8 +297,10 @@ Status build_hnsw_host(const float* rows, size_t n, int dim, int dist_func, cons
   g.total = (uint32_t)n;
   g.dim = dim;
   g.maxM = bp.maxM;
+  g.M = bp.M;
   g.maxM0 = bp.maxM0;
   g.maxlevel = b.maxlevel;
+  g.levels.assign(b.level.begin(), b.level.end());
   g.enterpoint = (uint32_t)b.enterpoint;
   g.dist_func = dist_func;
   g.ext_ids.assign(ext_ids, ext_ids + n);

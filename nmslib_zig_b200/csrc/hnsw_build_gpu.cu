@@ -483,8 +483,10 @@ Status build_hnsw_device(const float* d_rows, size_t n, int dim, int row_words, 
   g.total = (uint32_t)n;
   g.dim = dim;
   g.maxM = bp.maxM;
+  g.M = bp.M;
   g.maxM0 = bp.maxM0;
   g.maxlevel = maxlevel;
+  g.levels.assign(level.begin(), level.end());
   g.enterpoint = (uint32_t)enterpoint;
   g.dist_func = dist_func;
   g.ext_ids.assign(ext_ids, ext_ids + n);

@@ -57,12 +57,14 @@ Status read_regular(FILE* f, HnswGraph* out) {
   g.maxM = (int)maxM;
   g.maxM0 = (int)maxM0;
   g.maxlevel = maxlevel;
+  g.M = (int)M;
   g.enterpoint = enterpoint;
   g.dist_func = 0;
   g.links0.assign((size_t)total * g.maxM0, -1);
   g.links0_cnt.assign(total, 0);
   g.upper_off.assign(total, -1);
-  std::vector<int32_t> levels(total, 0);
+  std::vector<int32_t>& levels = g.levels;
+  levels.assign(total, 0);
   std::vector<int32_t> ids;
   for (uint32_t i = 0; i < total; ++i) {
     uint32_t level = 0;
@@ -92,7 +94,8 @@ Status read_regular(FILE* f, HnswGraph* out) {
   // level consistency (see read_hnsw_file): the descent follows a level-l link only into nodes that have level l
   if (total > 0 && levels[enterpoint] < maxlevel) {
     // (hnsw.cc:824-828 notes that maxlevel_ may exceed the entry node's level; the pointer search starts from
-    //  enterpoint_->level, hnsw.cc:1183, so that is the level the descent must use)
+    //  enterpoint_->level, hnsw.cc:1183, so that is the level the descent must use; a save writes the header's)
+    g.file_maxlevel = maxlevel;
     g.maxlevel = levels[enterpoint];
   }
   for (uint32_t i = 0; i < total; ++i)
@@ -182,7 +185,8 @@ Status read_hnsw_file(const std::string& path, HnswGraph* out) {
   // outside the upper-level block.
   if (maxlevel < 0) return Status::Err(kErrIO, "negative HNSW maxlevel");
   {
-    std::vector<int32_t> levels(total, 0);
+    std::vector<int32_t>& levels = g.levels;
+    levels.assign(total, 0);
     // (the blocks were appended in node order: a node's block ends where the next non-empty one starts)
     int64_t prev = -1;
     uint32_t prev_i = 0;
@@ -203,6 +207,27 @@ Status read_hnsw_file(const std::string& path, HnswGraph* out) {
       }
   }
   *out = std::move(g);
+  return Status::OK();
+}
+
+Status write_regular(const std::string& path, const HnswGraph& g) {
+  if (g.levels.size() != g.total || g.M <= 0) return Status::Err(kErrIO, "graph without levels or M: no regular file");
+  FilePtr f(fopen(path.c_str(), "wb"));
+  if (!f) return Status::Err(kErrIO, "cannot open " + path + " for writing");
+  bool ok = wr<uint32_t>(f.get(), 0) && wr<uint32_t>(f.get(), g.total) &&
+            wr<int32_t>(f.get(), g.file_maxlevel >= 0 ? g.file_maxlevel : g.maxlevel) &&
+            wr<uint32_t>(f.get(), g.enterpoint) && wr<uint64_t>(f.get(), (uint64_t)g.M) &&
+            wr<uint64_t>(f.get(), (uint64_t)g.maxM) && wr<uint64_t>(f.get(), (uint64_t)g.maxM0);
+  for (uint32_t i = 0; ok && i < g.total; ++i) {
+    const uint32_t level = (uint32_t)g.levels[i];
+    ok = wr<uint32_t>(f.get(), level);
+    for (uint32_t l = 0; ok && l <= level; ++l) {
+      const int32_t* lk = l == 0 ? &g.links0[(size_t)i * g.maxM0] : &g.upper[g.upper_off[i] + (size_t)(l - 1) * (g.maxM + 1)] + 1;
+      const uint32_t cnt = l == 0 ? (uint32_t)g.links0_cnt[i] : (uint32_t)lk[-1];
+      ok = wr<uint32_t>(f.get(), cnt) && (cnt == 0 || fwrite(lk, 4, cnt, f.get()) == cnt);
+    }
+  }
+  if (!ok) return Status::Err(kErrIO, "short write to " + path);
   return Status::OK();
 }
 

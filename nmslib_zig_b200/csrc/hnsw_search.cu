@@ -19,6 +19,10 @@
 // loads (lane c reads float4 c, c+32, ...), four neighbours in flight per warp; the
 // level-0 adjacency row (maxM0 ints) is one coalesced 128-byte read.  The kernel is
 // bound by HBM random-gather bandwidth, not FLOPs.
+// uint8 rows (l2sqr_sift, dist_kind 3) stay bytes: a 128-byte row is one word per lane, one coalesced
+// load per neighbour, and the distance is an exact integer (dp4a of byte differences, integer warp sum)
+// converted to float -- the value the widened fp32 sum gives, bit for bit, since every partial sum there
+// is an integer below 2^24.
 #include <algorithm>
 #include <cstdlib>
 
@@ -55,7 +59,7 @@ __device__ __forceinline__ void acc4(const float4& x, const float4& q, float& s)
   }
 }
 template <int KIND>
-__device__ __forceinline__ float fin_dist(float s) {
+__device__ __forceinline__ float fin_dist(float s) {  // (KIND 3 never gets here: evalG returns its integer sum)
   if constexpr (KIND == 0) return s;                                            // L2Sqr(16)Ext
   else if constexpr (KIND == 1) return fmaxf(0.f, 1.f - fmaxf(-1.f, fminf(1.f, s)));  // NormCosine hnsw.cc:78-81
   else return -s;                                                               // NegativeDotProduct :70-73
@@ -64,15 +68,41 @@ __device__ __forceinline__ float fin_dist(float s) {
 // distances of up to G nodes (t[g] valid for g < cnt) to the query in shared memory: G independent row
 // gathers in flight per lane and loop iteration (the kernel waits on these loads ~80 % of the time, ncu)
 template <int KIND, int G>
-__device__ __forceinline__ void evalG(const float* __restrict__ vectors, int row_words,
+__device__ __forceinline__ void evalG(const void* __restrict__ vectors, int row_words,
                                       const float4* __restrict__ q4, const int (&t)[G], int cnt, int lane,
                                       float (&out)[G]) {
+  if constexpr (KIND == 3) {
+    // byte rows: word c of a row holds elements 4c..4c+3; |x - q|^2 of one word is dp4a(|x - q|, |x - q|) per byte
+    // (at most 4 * 255^2), the row's sum at most 128 * 255^2 < 2^24, so the float conversion is exact
+    const uint32_t* xw[G];
+    uint32_t s[G];
+#pragma unroll
+    for (int g = 0; g < G; ++g) {
+      xw[g] = static_cast<const uint32_t*>(vectors) + (size_t)t[g < cnt ? g : 0] * row_words;
+      s[g] = 0u;
+    }
+    const uint32_t* qw = reinterpret_cast<const uint32_t*>(q4);
+    for (int c = lane; c < row_words; c += 32) {
+      uint32_t a[G];
+#pragma unroll
+      for (int g = 0; g < G; ++g) a[g] = g < cnt ? __ldg(xw[g] + c) : 0u;
+      const uint32_t q = qw[c];
+#pragma unroll
+      for (int g = 0; g < G; ++g) {
+        const uint32_t d = __vabsdiffu4(a[g], q);
+        s[g] = __dp4a(d, d, s[g]);
+      }
+    }
+#pragma unroll
+    for (int g = 0; g < G; ++g) out[g] = (float)__reduce_add_sync(FULL, s[g]);
+    return;
+  }
   const int rw4 = row_words >> 2;
   const float4* x[G];
   float s[G];
 #pragma unroll
   for (int g = 0; g < G; ++g) {
-    x[g] = reinterpret_cast<const float4*>(vectors + (size_t)t[g < cnt ? g : 0] * row_words);
+    x[g] = reinterpret_cast<const float4*>(static_cast<const float*>(vectors) + (size_t)t[g < cnt ? g : 0] * row_words);
     s[g] = 0.f;
   }
   if (cnt == G) {
@@ -120,7 +150,7 @@ __device__ __forceinline__ uint64_t warp_sort64(uint64_t v, int lane) {
 
 // ---- pieces shared by the one-warp kernel and the team kernel (one warp executes each of them) ----------------
 
-// stage the query in shared memory (cosine: NormalizeVect, hnsw.h:486-497)
+// stage the query in shared memory (cosine: NormalizeVect, hnsw.h:486-497; byte rows: the words are copied as they are)
 template <int KIND>
 __device__ __forceinline__ void stage_query(const float* __restrict__ qsrc, float* qv, int row_words, int lane) {
   float ss = 0.f;
@@ -273,7 +303,7 @@ __device__ __forceinline__ void beam_advance(const int* wdat, int n_w, int lane,
 
 template <int KIND, int EVG, int MINB>  // EVG: neighbour vectors gathered at once per warp
 __global__ void __launch_bounds__(WARPS * 32, MINB)
-hnsw_search_kernel(HnswDeviceGraph g, const float* __restrict__ queries, int nq, int k, int ef, int cap,
+hnsw_search_kernel(HnswDeviceGraph g, const void* __restrict__ queries, int nq, int k, int ef, int cap,
                    int cap_r, uint8_t* __restrict__ visited, size_t visited_stride,
                    int* __restrict__ slot_epoch, uint64_t* __restrict__ out_keys,
                    unsigned long long* __restrict__ counters) {
@@ -310,7 +340,7 @@ hnsw_search_kernel(HnswDeviceGraph g, const float* __restrict__ queries, int nq,
     const uint8_t ep = (uint8_t)epoch;
     __syncwarp();
 
-    stage_query<KIND>(queries + (size_t)qi * g.row_words, qv, g.row_words, lane);
+    stage_query<KIND>(static_cast<const float*>(queries) + (size_t)qi * g.row_words, qv, g.row_words, lane);
     int cur_node;
     float cur_dist;
     greedy_descent<KIND, EVG>(g, q4, lane, cur_node, cur_dist, n_eval);
@@ -401,7 +431,7 @@ __device__ __forceinline__ void team_sync(int team) {
 
 template <int KIND, int EVG, int TW>
 __global__ void __launch_bounds__(WARPS * 32, 6)
-hnsw_search_team_kernel(HnswDeviceGraph g, const float* __restrict__ queries, int nq, int k, int ef, int cap,
+hnsw_search_team_kernel(HnswDeviceGraph g, const void* __restrict__ queries, int nq, int k, int ef, int cap,
                         int cap_r, uint8_t* __restrict__ visited, size_t visited_stride,
                         int* __restrict__ slot_epoch, uint64_t* __restrict__ out_keys,
                         unsigned long long* __restrict__ counters) {
@@ -472,7 +502,7 @@ hnsw_search_team_kernel(HnswDeviceGraph g, const float* __restrict__ queries, in
     int n_w = 1, cur = 0;
     if (warp == 0) {
       // query staging and greedy descent by the team's warp 0 alone: the one-warp kernel's arithmetic
-      stage_query<KIND>(queries + (size_t)qi * g.row_words, qv, g.row_words, lane);
+      stage_query<KIND>(static_cast<const float*>(queries) + (size_t)qi * g.row_words, qv, g.row_words, lane);
       int cur_node;
       float cur_dist;
       greedy_descent<KIND, EVG>(g, q4, lane, cur_node, cur_dist, n_eval);
@@ -562,7 +592,7 @@ hnsw_search_team_kernel(HnswDeviceGraph g, const float* __restrict__ queries, in
 int hnsw_max_ef() { return MAX_EF; }
 int hnsw_warps_per_block() { return WARPS; }
 
-cudaError_t launch_hnsw_search(const HnswDeviceGraph& g, const float* queries, int nq, int k, int ef,
+cudaError_t launch_hnsw_search(const HnswDeviceGraph& g, const void* queries, int nq, int k, int ef,
                                uint8_t* visited, int* slot_epoch, int slots, uint64_t* out_keys,
                                unsigned long long* counters, cudaStream_t stream) {
   if (nq <= 0) return cudaSuccess;
@@ -623,6 +653,7 @@ cudaError_t launch_hnsw_search(const HnswDeviceGraph& g, const float* queries, i
         case 0: NB_TEAM2(0); break;
         case 1: NB_TEAM2(1); break;
         case 2: NB_TEAM2(2); break;
+        case 3: NB_TEAM2(3); break;
         default: return cudaErrorInvalidValue;
       }
 #undef NB_TEAM2
@@ -652,6 +683,7 @@ cudaError_t launch_hnsw_search(const HnswDeviceGraph& g, const float* queries, i
     case 0: NB_HNSW(0); break;
     case 1: NB_HNSW(1); break;
     case 2: NB_HNSW(2); break;
+    case 3: NB_HNSW(3); break;
     default: return cudaErrorInvalidValue;
   }
 #undef NB_HNSW

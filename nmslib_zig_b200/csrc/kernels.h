@@ -182,19 +182,20 @@ cudaError_t launch_range_verify(const float* db, const float* queries, const int
 
 // ---- hnsw_search.cu ------------------------------------------------------------------
 struct HnswDeviceGraph {
-  const float* vectors;      // [n][row_words] (cosine: unit-norm rows, as the reference stores them)
+  const void* vectors;       // [n][row_words] words: float32 (cosine: unit-norm rows, as the reference stores them)
+                             // or, dist_kind 3, packed uint8 rows
   const int32_t* links0;     // [n][maxM0]
   const int32_t* links0_cnt; // [n]
   const int32_t* upper;      // concatenated upper-level lists: per level (maxM+1) ints, count first
   const int64_t* upper_off;  // [n] offset into `upper`, -1 when the node lives on level 0 only
   const int32_t* ext_ids;    // [n]
   int n, dim, row_words, maxM, maxM0, maxlevel, enterpoint;
-  int dist_kind;             // 0 squared L2, 1 cosine on unit vectors, 2 negative dot product
+  int dist_kind;             // 0 squared L2, 1 cosine on unit vectors, 2 negative dot product, 3 squared L2 of uint8 rows
 };
-// One warp per query.  visited: [slots][n] epoch bytes, epochs: [slots] current epoch.
-// out_keys: [nq][k] (ordered(distance) << 32 | internal position), counters: [2] atomics
-// (distance evaluations, expansions), may be NULL.
-cudaError_t launch_hnsw_search(const HnswDeviceGraph& g, const float* queries, int nq, int k, int ef,
+// One warp per query.  queries: [nq][row_words] words laid out like the rows.  visited: [slots][n] epoch bytes,
+// epochs: [slots] current epoch.  out_keys: [nq][k] (ordered(distance) << 32 | internal position), counters: [2]
+// atomics (distance evaluations, expansions), may be NULL.
+cudaError_t launch_hnsw_search(const HnswDeviceGraph& g, const void* queries, int nq, int k, int ef,
                                uint8_t* visited, int* slot_epoch, int slots, uint64_t* out_keys,
                                unsigned long long* counters, cudaStream_t stream);
 int hnsw_max_ef();

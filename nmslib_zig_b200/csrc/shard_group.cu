@@ -242,7 +242,8 @@ Status ShardGroup::prepare(Engine* host, size_t nq, size_t k) {
     Status gs = host->ensure_graph();  // built once (on the device when the parameters say so), or imported
     if (!gs.ok()) return gs;
     host->release_device();            // (the handle's engine stays the host store; the replicas hold the device copies)
-    const float* rows = host->hnsw_rows_for_save();
+    // (float: the search-ready rows, cosine normalised; uint8: the host store's byte rows, which the search reads)
+    const void* rows = host->is_u8() ? (const void*)host->row_u8(0) : (const void*)host->hnsw_rows_for_save();
     const size_t G = m.devices.size();
     m.shards.clear();
     m.shards.resize(G);

@@ -527,7 +527,8 @@ class Index:
 
     def knnDevice(self, d_queries_ptr: int, nq: int, dim: int, k: int, d_ids_ptr: int, d_dists_ptr: int,
                   d_keys_ptr: int = 0, stream: int = 0):
-        """Device-resident query: raw device pointers (e.g. torch.Tensor.data_ptr())."""
+        """Device-resident query: raw device pointers (e.g. torch.Tensor.data_ptr()); the queries are float32, or
+        uint8 for a DenseUInt8Vector index (seq_search or hnsw)."""
         _check(lib().nmslib_b200_knn_device(self.handle, d_queries_ptr, nq, dim, k, d_ids_ptr, d_dists_ptr,
                                             d_keys_ptr or None, stream or None))
 
