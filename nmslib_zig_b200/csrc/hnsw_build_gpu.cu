@@ -23,7 +23,8 @@
 // result is searched by hnsw_search.cu, saved by nmslib_save_index and loadable by the reference.
 // The graph is NOT the reference's graph (neither is the reference's own from run to run, SURVEY 0.7): it is
 // held to recall parity -- recall@10 at a given efSearch at or above a reference-built graph
-// (tests/test_hnsw_gpu.py, tools/hnsw_bench.py --build device).
+// (tests/test_hnsw_gpu.py, tools/hnsw_bench.py --build device).  On rows whose distances are exact fp32 values the
+// build is deterministic, and tests/test_hnsw_build_exact_gpu.py holds it to a restatement list for list.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -45,6 +46,7 @@ constexpr int HB_MAXC = 256;    // candidates per new point (<= the scan's max k
 constexpr int HB_MAXKEEP = 64;  // M, maxM, maxM0 <= 64
 constexpr int HB_MAXIN = 32;    // back links taken per neighbour and batch (closest first)
 constexpr int HB_WARPS = 4;
+static_assert(HB_MAXIN <= 32, "hb_link_kernel reads one incoming link per lane");
 
 // distance of the graph: 0 squared L2, 1 cosine on unit rows, 2 negative dot (hnsw_search.cu uses the same kinds)
 template <int KIND>
@@ -222,10 +224,11 @@ hb_link_kernel(const float* __restrict__ rows, int row_words, const uint64_t* __
   if (w >= *seg_count) return;
   const int s0 = seg_start[w];
   const uint32_t c = (uint32_t)(rkey[s0] >> 32);
-  // incoming links: the run is sorted by distance, the first HB_MAXIN are the closest
+  // incoming links: the run is sorted by distance, the first HB_MAXIN are the closest (the shared lists above hold
+  // no more, whatever the warp width)
   uint64_t key = KEY_MAX;
   if (s0 + lane < total) key = rkey[s0 + lane];
-  const bool in_ok = key != KEY_MAX && (uint32_t)(key >> 32) == c;
+  const bool in_ok = lane < HB_MAXIN && key != KEY_MAX && (uint32_t)(key >> 32) == c;
   const unsigned bal = __ballot_sync(FULLW, in_ok);  // a prefix of the lanes (the run is contiguous)
   const int inc = __popc(bal);
   const int have = cnt[c];
